@@ -13,7 +13,9 @@ reward, done, auto-reset).
 
 Prints ONE JSON line (rank 0).  `value` = whole-job env-steps/s with actions resident
 in HBM; `e2e` = the same through auv_step_host with host buffers (H2D actions, D2H
-obs/reward/done inside the timed region).
+obs/reward/done inside the timed region).  `--dump-outputs DIR` also writes what the last
+timed step returned as DIR/<name>.npy (see dump_outputs): the inputs depend only on the
+arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -119,6 +121,9 @@ def parse():
                          "episodes desynchronised); also gives the clock sampler its samples under load")
     ap.add_argument("--scenario-cache", default=None,
                     help="pickle the generated scenario set here / reuse it (tuning sweeps; same seeds => same set)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what AUVVecEnv.step returned in the last timed step as DIR/<name>.npy (rank 0, float32), "
+                         "to compare two builds output for output; see dump_outputs")
     return ap.parse_args()
 
 
@@ -390,6 +395,32 @@ def roofline_block(N, R, obs_dim, step_ms, kernel_ms, records_per_step, seg_test
     return roof
 
 
+DUMP_BYTES = 60 << 20  # array data of --dump-outputs; with the .npy headers the directory stays under 64 MB
+
+
+def dump_outputs(out_dir, step_result):
+    """Write the (obs, reward, done, info) tuple of AUVVecEnv.step as out_dir/<name>.npy, every array as float32
+    (done / collision / reached_goal as 0.0 / 1.0), one row per env.  When all rows exceed DUMP_BYTES, every array
+    keeps the same rows: a sorted sample drawn with a fixed seed, so that two runs with the same arguments write the
+    same envs."""
+    import torch
+
+    obs, reward, done, info = step_result
+    arrays = {"obs": obs, "reward": reward, "done": done, **info}
+    n = obs.shape[0]
+    row_bytes = 4 * sum(a[0].numel() for a in arrays.values())
+    keep = min(n, DUMP_BYTES // row_bytes)
+    rows = None
+    if keep < n:
+        rows = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, keep, replace=False))).to(obs.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if rows is not None:
+            a = a.index_select(0, rows)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.to(torch.float32).cpu().numpy())
+    return keep
+
+
 # --------------------------------------------------------------------------------------
 # GPU arm
 # --------------------------------------------------------------------------------------
@@ -455,12 +486,13 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     step_no = [0]
+    last_step = [None]  # what the latest AUVVecEnv.step returned (views of the env's output buffers)
 
     def run_steps(k):
         """k steps through the public API (AUVVecEnv.step), scenario refresh included"""
         for _ in range(k):
             i = step_no[0]
-            env.step(actions[i % n_act])
+            last_step[0] = env.step(actions[i % n_act])
             if fresh and i % args.refresh_every == args.refresh_every - 1:
                 env.refresh_finished_device(seed=seed)
             step_no[0] = i + 1
@@ -501,6 +533,9 @@ def run_ours(args):
     dones_per_step = stats_timed["episodes"] / max(K, 1) / world
     steady_records = float(env._scratch["rec_cnt"].sum().item()) / N
     cross_track = float(env._st["nav"][:, 2].abs().mean().item())
+    dumped_rows = None
+    if args.dump_outputs and rank == 0:  # before the legs below step the env again
+        dumped_rows = dump_outputs(args.dump_outputs, last_step[0])
 
     # ---- per-kernel attribution: K more steps of the same steady state on ONE stream with CUDA events
     #      around each kernel (auv_step_timed); these are the launch durations the roofline uses
@@ -688,6 +723,8 @@ def run_ours(args):
         "roofline": roof,
         "episode_stats": stats_timed,
     }
+    if dumped_rows is not None:
+        line["outputs_dumped"] = {"dir": args.dump_outputs, "envs": dumped_rows, "of": N}
     if not args.no_cpu_baseline and world == 1:  # reported on rank 0 at N=1 only
         small = argparse.Namespace(**vars(args))
         small.envs = args.cpu_sample_envs

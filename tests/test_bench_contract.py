@@ -1,11 +1,16 @@
-"""bench.py contract checks that run without a GPU: the flags the driver passes parse, and the
-reference arm (CPU oracle port) prints exactly one JSON line with the keys the driver reads."""
+"""bench.py contract checks: the reference arm (CPU oracle port) prints exactly one JSON line with the
+contract keys, the GPU arm refuses to run without CUDA, the roofline assembly, and --dump-outputs (its
+host logic on the CPU, its repeatability on the GPU)."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+OUTPUT_NAMES = {"obs", "reward", "done", "collision", "reached_goal", "goal_distance", "progress", "terminal_observation"}
 
 
 def test_reference_arm_prints_one_json_line_with_the_contract_keys():
@@ -30,8 +35,6 @@ def test_reference_arm_is_silent_on_other_ranks():
 
 
 def test_gpu_arm_fails_loudly_without_cuda():
-    import pytest
-
     torch = pytest.importorskip("torch")
     if torch.cuda.is_available():
         pytest.skip("CUDA present")
@@ -73,3 +76,54 @@ def test_roofline_block_names_the_longest_single_launch():
     import json
 
     json.dumps(r)  # serialisable
+
+
+def test_dump_outputs_writes_the_step_tuple_as_float32_and_samples_the_same_rows(tmp_path, monkeypatch):
+    """bench.dump_outputs: one float32 .npy per array of AUVVecEnv.step's (obs, reward, done, info); above the byte
+    budget every array keeps the same seeded sample of env rows.  CPU tensors stand in for the device buffers."""
+    torch = pytest.importorskip("torch")
+    import bench
+
+    n, d = 1000, 186
+    g = torch.Generator().manual_seed(3)
+    obs = torch.rand((n, d), generator=g)
+    flag = lambda: (torch.rand(n, generator=g) < 0.3).to(torch.uint8)
+    info = dict(collision=flag(), reached_goal=flag(), goal_distance=torch.rand(n, generator=g),
+                progress=torch.rand(n, generator=g), terminal_observation=torch.rand((n, d), generator=g))
+    step = (obs, torch.rand(n, generator=g), flag(), info)
+
+    assert bench.dump_outputs(str(tmp_path / "all"), step) == n
+    out = {k: np.load(tmp_path / "all" / f"{k}.npy") for k in OUTPUT_NAMES}
+    assert set(os.listdir(tmp_path / "all")) == {f"{k}.npy" for k in OUTPUT_NAMES}
+    assert all(a.dtype == np.float32 and a.shape[0] == n for a in out.values())
+    assert np.array_equal(out["obs"], obs.numpy()) and np.array_equal(out["done"], step[2].numpy().astype(np.float32))
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4 * 100 * (2 * d + 6))
+    assert bench.dump_outputs(str(tmp_path / "a"), step) == 100
+    assert bench.dump_outputs(str(tmp_path / "b"), step) == 100
+    a = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in OUTPUT_NAMES}
+    b = {k: np.load(tmp_path / "b" / f"{k}.npy") for k in OUTPUT_NAMES}
+    assert all(np.array_equal(a[k], b[k]) and a[k].shape[0] == 100 for k in OUTPUT_NAMES)
+    rows = np.flatnonzero(np.isin(obs.numpy()[:, 0], a["obs"][:, 0]))  # the sampled env rows, in order
+    assert len(rows) == 100
+    assert np.array_equal(a["obs"], obs.numpy()[rows]) and np.array_equal(a["progress"], info["progress"].numpy()[rows])
+    assert np.array_equal(a["terminal_observation"], info["terminal_observation"].numpy()[rows])
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_repeat_with_the_same_arguments(tmp_path):
+    """Two bench.py runs with the same arguments time --steps steps and write the same outputs of the last one."""
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "7", "--warmup", "3", "--envs", "512",
+           "--n-paths", "64", "--preroll-steps", "60", "--no-cpu-baseline", "--no-e2e"]
+    for run in ("a", "b"):
+        res = subprocess.run(cmd + ["--dump-outputs", str(tmp_path / run)], capture_output=True, text=True, timeout=600,
+                             cwd=ROOT)
+        assert res.returncode == 0, res.stderr[-2000:]
+        d = json.loads(res.stdout.strip())
+        assert d["steps"] == 7 and d["outputs_dumped"] == {"dir": str(tmp_path / run), "envs": 512, "of": 512}
+    a = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in OUTPUT_NAMES}
+    b = {k: np.load(tmp_path / "b" / f"{k}.npy") for k in OUTPUT_NAMES}
+    assert a["obs"].shape == (512, 186) and all(v.dtype == np.float32 for v in a.values())
+    assert np.abs(a["obs"]).max() > 0
+    for k in OUTPUT_NAMES:
+        assert np.array_equal(a[k], b[k]), k
