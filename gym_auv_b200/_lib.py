@@ -8,7 +8,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("AUV_B200_LIB", os.path.join(_HERE, "libauv_b200.so"))  # override: tuning builds only
-ABI_VERSION = 19
+ABI_VERSION = 20
 REC_BYTES = 80
 MAX_POLY_VERTS = 192
 STATUS_REC_OVERFLOW = 1
@@ -101,6 +101,8 @@ class AuvPathBank(C.Structure):
         ("sb_chord", _vp),
         ("sb_dev", _vp),
         ("pp", _vp),
+        ("sub_chord", _vp),
+        ("sub_dev", _vp),
     ]
 
 
@@ -218,7 +220,8 @@ class AuvRefreshScratch(C.Structure):
 
 class AuvPathBuild(C.Structure):
     _fields_ = [("hdr", _vp), ("poly_xy", _vp), ("poly_cum", _vp), ("poly_f32", _vp), ("blk_chord", _vp), ("blk_dev", _vp),
-                ("sb_chord", _vp), ("sb_dev", _vp), ("pp", _vp), ("n_knots", C.c_int32), ("vcap", C.c_int32)]
+                ("sb_chord", _vp), ("sb_dev", _vp), ("pp", _vp), ("n_knots", C.c_int32), ("vcap", C.c_int32),
+                ("sub_chord", _vp), ("sub_dev", _vp)]
 
 
 class AuvCompact(C.Structure):

@@ -1728,6 +1728,8 @@ static int launch_vessel_nav(const AuvConfig* cfg, const AuvRayTable* rays, cons
                              const AuvScenarioPool* pool, AuvBatch* batch, AuvStepOut* out,
                              const float* actions, void* stream, int e0 = 0, int cnt = -1, bool with_obstacles = false,
                              cudaEvent_t between = nullptr /* recorded between the two launches (auv_step_timed) */) {
+  if ((paths->sub_chord == nullptr) != (paths->sub_dev == nullptr))
+    return set_err(AUV_EINVAL, "paths: sub_chord and sub_dev are both set or both NULL");
   if (cnt < 0) cnt = batch->n_envs - e0;
   const int per_cta = AUV_NAV_THREADS / AUV_NAV_G;  // envs per CTA
   const int blocks = (cnt + per_cta - 1) / per_cta;
@@ -2405,8 +2407,10 @@ int auv_pathbank_build(const double* waypoints, const int32_t* n_wp, const int32
       !out->sb_dev || !out->pp)
     return set_err(AUV_EINVAL, "AuvPathBuild holds a NULL array");
   if (out->n_knots != auv::PB_NK) return set_err(AUV_EINVAL, "n_knots must be 1000");
-  if (out->vcap <= 0 || out->vcap % (AUV_PATH_BLOCK * AUV_PATH_SUPER) != 0)
-    return set_err(AUV_EINVAL, "vcap must be a positive multiple of AUV_PATH_BLOCK * AUV_PATH_SUPER");
+  if ((out->sub_chord == nullptr) != (out->sub_dev == nullptr))
+    return set_err(AUV_EINVAL, "AuvPathBuild: sub_chord and sub_dev are both set or both NULL");
+  if (out->vcap <= 0 || out->vcap % (2 * AUV_PATH_BLOCK * AUV_PATH_SUPER) != 0)
+    return set_err(AUV_EINVAL, "vcap must be a positive multiple of 2 * AUV_PATH_BLOCK * AUV_PATH_SUPER");
   const size_t smem = auv::pathbuild_smem_bytes();
   static std::atomic<int> configured[64];
   int dev = 0;
@@ -2428,6 +2432,8 @@ int auv_pathbank_build(const double* waypoints, const int32_t* n_wp, const int32
   o.sb_dev = out->sb_dev;
   o.pp = out->pp;
   o.vcap = out->vcap;
+  o.sub_chord = out->sub_chord;
+  o.sub_dev = out->sub_dev;
   auv::k_path_build<<<n, auv::PB_THREADS, smem, (cudaStream_t)stream>>>(waypoints, n_wp, path_ids, n, o, status);
   return cuda_check(cudaGetLastError(), "k_path_build");
 }

@@ -100,21 +100,6 @@ __device__ __forceinline__ double seg_d2(double px, double py, double2 A, double
   return cr * cr / len2;
 }
 
-// FP32 squared distance from the origin-relative point (qx, qy) to segment AB (same case split)
-__device__ __forceinline__ float seg_d2_f(float qx, float qy, float2 A, float2 B) {
-  const float ex = B.x - A.x, ey = B.y - A.y;
-  const float wx = qx - A.x, wy = qy - A.y;
-  const float len2 = ex * ex + ey * ey;
-  const float num = wx * ex + wy * ey;
-  if (len2 == 0.f || num <= 0.f) return wx * wx + wy * wy;
-  if (num >= len2) {
-    const float zx = qx - B.x, zy = qy - B.y;
-    return zx * zx + zy * zy;
-  }
-  const float cr = wx * ey - wy * ex;
-  return cr * cr / len2;
-}
-
 // the same distance as the exact fraction num / den (den > 0): candidates are compared by cross-multiplication,
 // one division for the winner instead of one per segment (FP64 divisions are ~20 instructions each)
 __device__ __forceinline__ void seg_d2_frac(double px, double py, double2 A, double2 B, double& num, double& den) {
@@ -153,9 +138,6 @@ __device__ __forceinline__ unsigned group_ballot(unsigned gm, int lane, bool pre
   return G == 32 ? b : ((b >> (lane & ~(G - 1))) & ((1u << G) - 1u));
 }
 
-// upper bound of |coordinate| of a path's origin-relative polyline (stored in the header's spare double)
-__device__ __forceinline__ float h_extent(const AuvPathHdr& h) { return (float)h.extent; }
-
 // capsule tables of one path: the global arrays, or the CTA's shared-memory copy of them
 struct PathTabs {
   const float4* sbc;    // superblock chords
@@ -164,17 +146,21 @@ struct PathTabs {
   const float2* aux;    // block (1/|e|^2, deviation)
 };
 
-// GEOS LengthIndexOfPoint::indexOf (LineString.project) restated as an exact three-level
-// search, executed by a GROUP of G lanes per env.  Level 2 = superblocks of AUV_PATH_SUPER
-// blocks, level 1 = blocks of 32 segments; each node is a capsule (chord, max deviation) that
-// contains its part of the polyline, so
+constexpr int kSubPerBlk = AUV_PATH_BLOCK / AUV_PATH_SUB;  // sub-blocks of a block
+
+// GEOS LengthIndexOfPoint::indexOf (LineString.project) restated as an exact four-level
+// search, executed by a GROUP of G lanes per env.  Level 3 = superblocks of AUV_PATH_SUPER
+// blocks, level 2 = blocks of 32 segments, level 1 = sub-blocks of AUV_PATH_SUB segments; each
+// node is a capsule (chord, max deviation) that contains its part of the polyline, so
 //   dist(P, node) in [dc - dev, dc + dev],  dc = dist(P, chord)   (FP32, padded).
 // An upper bound `ub` of the minimum distance comes either from the segment the previous step's
 // projection ended on (WARM: the own-ship moves < 1 m per step, so the exact FP64 distance to a few
 // segments around it is within millimetres of the answer -- it is only used as a bound, the search
 // below stays exhaustive) or, without one (first step of an episode), from pass A over the
 // superblock capsules and pass B over the block capsules of the surviving superblocks.  Pass C
-// refines in FP64 every block whose lower bound does not exceed `ub`.  In every pass the lanes of
+// tests the sub-block capsules of every block whose lower bound does not exceed `ub` and refines
+// the surviving sub-blocks in FP64 (a segment d along the path from the foot point is ~d^2 / 2r farther
+// away at cross-track distance r, so these are the one or two sub-blocks around it).  In every pass the lanes of
 // the group take different nodes / segments, so one round of loads covers G of them, and bounds are
 // shared by shuffle-min; all bounds are compared in the squared domain.  Every loop pops the next set
 // bit of a mask that is uniform in the group ("by rank"): the groups of a warp then run their r-th
@@ -230,18 +216,13 @@ __device__ __noinline__ float project_cold_bound(const PathTabs& T, const int nb
   return ub;
 }
 
-#ifndef AUV_PROJ_UNROLL
-#define AUV_PROJ_UNROLL 2  // unroll of the FP64 refine over a lane's 8 segments (1 / 4 / 8 measured: see DESIGN 5d)
-#endif
-constexpr int kProjUnroll = AUV_PROJ_UNROLL;
 template <int G>
 __device__ AUV_PROJECT_INLINE double project_group(const AuvPathBank& pb, const AuvPathHdr& h, const PathTabs& T,
                                                    const double px, const double py, const int prev_seg,
                                                    const int lane, const unsigned gm, int& seg_out, int* status = nullptr) {
   constexpr int KB = AUV_PATH_SUPER / G;  // blocks of a superblock per lane
-  constexpr int KS = AUV_PATH_BLOCK / G;  // segments of a block per lane
-  constexpr int KBB = KB < 8 ? KB : 8;    // ... loaded in batches of at most 8
-  constexpr int KSB = KS < 8 ? KS : 8;
+  constexpr int SPL = AUV_PATH_SUB > G ? AUV_PATH_SUB / G : 1;  // segments of a sub-block per lane
+  static_assert(G >= kSubPerBlk, "one lane per sub-block of a block");
   const int sub = lane & (G - 1);
   const int nseg = h.nseg;
   const int nblk = (nseg + AUV_PATH_BLOCK - 1) / AUV_PATH_BLOCK;
@@ -253,23 +234,19 @@ __device__ AUV_PROJECT_INLINE double project_group(const AuvPathBank& pb, const 
   const float4* sbc = T.sbc;
   const float2* sba = T.sba;
   const double2* __restrict__ poly = reinterpret_cast<const double2*>(pb.poly_xy) + h.v0;
-  const float2* __restrict__ polyf = reinterpret_cast<const float2*>(pb.poly_f32) + h.v0;
+  const float4* __restrict__ subc = reinterpret_cast<const float4*>(pb.sub_chord) + kSubPerBlk * h.b0;
+  const float2* __restrict__ subd = reinterpret_cast<const float2*>(pb.sub_dev) + kSubPerBlk * h.b0;
   const float up = 1.f + 4e-6f, dn2 = (1.f - 4e-6f) * (1.f - 4e-6f);
-  // error bound of an FP32 point-segment distance on the origin-relative FP32 polyline: vertex and query
-  // rounding (half an ulp of the coordinate magnitude each) plus the arithmetic, generously
-  const float ftol = 4e-7f * (fabsf(qx) + fabsf(qy) + h_extent(h)) + 5e-5f;
   float ub = INFINITY;
 #define AUV_TIGHTEN(d2, dv)                                         \
   if ((d2) < ub * ub) ub = fminf(ub, sqrtf(d2) * up + (dv) + pad);
 #define AUV_PRUNED(d2, dv) ((d2) * dn2 > (ub + (dv) + pad) * (ub + (dv) + pad))
   const bool warm = prev_seg >= 0 && prev_seg < nseg;  // uniform in the group
   if (warm) {
-    // lanes look at segments prev-3, prev, prev+3, prev+6 (...): an actual segment's distance (FP32 copy
-    // of the polyline, padded by its error bound ftol)
+    // lanes look at segments prev-3, prev, prev+3, prev+6 (...): an actual segment's exact distance
+    // (FP64; rounding to FP32 is covered by `up`)
     const int k = min(max(prev_seg + (sub - 1) * 3, 0), nseg - 1);
-    float d2 = seg_d2_f(qx, qy, polyf[k], polyf[k + 1]);
-    d2 = group_min<G>(gm, d2);
-    ub = sqrtf(d2) * up + ftol + pad;
+    ub = sqrtf(group_min<G>(gm, (float)seg_d2(px, py, poly[k], poly[k + 1]))) * up + pad;
   } else {
     ub = project_cold_bound<G>(T, nblk, nsb, qx, qy, pad, lane, gm);  // first step of an episode: out of line
   }
@@ -306,25 +283,39 @@ __device__ AUV_PROJECT_INLINE double project_group(const AuvPathBank& pb, const 
         const int b = sb * AUV_PATH_SUPER + __ffs(cand) - 1;
         cand &= cand - 1;
         const int se = min(nseg, (b + 1) * AUV_PATH_BLOCK);
-        const int k0 = b * AUV_PATH_BLOCK + sub * KS;  // this lane's consecutive segments
         AUV_CHECK(status, b >= 0 && b < nblk && sb < nsb);
-        // (screening these in FP32 first was measured slower: far from the path many segments tie within the
+        // the block's sub-block capsules, one per lane (without sub-block tables every sub-block is refined)
+        unsigned subs = (1u << kSubPerBlk) - 1u;  // bit = sub-block offset inside the block, uniform in the group
+        if (pb.sub_chord != nullptr) {
+          const int j = b * kSubPerBlk + min(sub, kSubPerBlk - 1);
+          const float4 ch = subc[j];
+          const float2 ax = subd[j];
+          subs = group_ballot<G>(gm, lane, sub < kSubPerBlk && j * AUV_PATH_SUB < nseg &&
+                                               !AUV_PRUNED(pt_chord_d2_f(qx, qy, ch, ax.x), ax.y));
+        }
+        // (screening segments in FP32 first was measured slower: far from the path many segments tie within the
         // FP32 error bound, and the divergent FP64 re-evaluation costs more than evaluating all of them)
-        double2 va = poly[min(k0, se)];
-#pragma unroll kProjUnroll
-        for (int u = 0; u < KS; ++u) {
-          const double2 vb = poly[min(k0 + u + 1, se)];
-          if (k0 + u < se) {
-            double num, den;
-            seg_d2_frac(px, py, va, vb, num, den);
-            // a lane's segments come in increasing order over the whole search: strictly smaller only
-            if (num * best_den < best_num * den) {
-              best_num = num;
-              best_den = den;
-              best_seg = k0 + u;
+        while (subs) {
+          const int j = b * kSubPerBlk + __ffs(subs) - 1;
+          subs &= subs - 1;
+          const int je = j * AUV_PATH_SUB + AUV_PATH_SUB;
+          const int k0 = j * AUV_PATH_SUB + sub * SPL;  // this lane's consecutive segments
+          double2 v[SPL + 1];
+#pragma unroll
+          for (int u = 0; u <= SPL; ++u) v[u] = poly[min(k0 + u, se)];
+#pragma unroll
+          for (int u = 0; u < SPL; ++u) {
+            if (k0 + u < min(se, je)) {
+              double num, den;
+              seg_d2_frac(px, py, v[u], v[u + 1], num, den);
+              // a lane's segments come in increasing order over the whole search: strictly smaller only
+              if (num * best_den < best_num * den) {
+                best_num = num;
+                best_den = den;
+                best_seg = k0 + u;
+              }
             }
           }
-          va = vb;
         }
       }
     }

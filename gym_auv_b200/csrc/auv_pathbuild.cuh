@@ -3,7 +3,8 @@
 //   3 x { chord-length parameter of the current points -> PCHIP (Fritsch-Carlson slopes) ->
 //         resample at linspace(0, arc[-1], 1000) }
 //   -> PPoly knots / coefficients, the 0.1 m polyline with its chord-length prefix sums, the FP32
-//      copy, and the capsule tables of the projection search -- the layout of AuvPathBank.
+//      copy, and the capsule tables of the projection search (sub-blocks, blocks, superblocks) -- the layout of
+//      AuvPathBank.
 // The arithmetic follows SciPy's evaluation order (scipy.interpolate.PchipInterpolator:
 // _find_derivatives / _edge_case, CubicHermiteSpline coefficients, _ppoly.evaluate_poly1's power
 // sum) and NumPy's linspace / cumsum, every operation an explicit round-to-nearest intrinsic (no
@@ -78,7 +79,9 @@ struct PathBuildOut {
   float* sb_chord;
   float* sb_dev;
   double* pp;
-  int vcap;  // vertices per path slot (a multiple of AUV_PATH_BLOCK * AUV_PATH_SUPER)
+  int vcap;  // vertices per path slot (a multiple of 2 * AUV_PATH_BLOCK * AUV_PATH_SUPER)
+  float* sub_chord;  // NULL: no sub-block tables
+  float* sub_dev;
 };
 __host__ __device__ constexpr size_t pathbuild_smem_bytes() {
   return sizeof(double) * (PB_NK + 2 * PB_NK + 2 * PB_NK + 2 * (PB_NK - 1) * 4) + 64;
@@ -278,6 +281,11 @@ __global__ void __launch_bounds__(PB_THREADS) k_path_build(const double* __restr
               reinterpret_cast<float2*>(out.blk_dev) + (size_t)p * bcap);
   pb_capsules(poly, ox, oy, nseg, AUV_PATH_BLOCK * AUV_PATH_SUPER, extent1,
               reinterpret_cast<float4*>(out.sb_chord) + (size_t)p * scap, reinterpret_cast<float2*>(out.sb_dev) + (size_t)p * scap);
+  if (out.sub_chord != nullptr) {
+    const int ucap = out.vcap / AUV_PATH_SUB;
+    pb_capsules(poly, ox, oy, nseg, AUV_PATH_SUB, extent1, reinterpret_cast<float4*>(out.sub_chord) + (size_t)p * ucap,
+                reinterpret_cast<float2*>(out.sub_dev) + (size_t)p * ucap);
+  }
   if (tid == 0) {
     AuvPathHdr h;
     h.v0 = (int)v0;

@@ -7,7 +7,7 @@ per distinct path, exactly the tables the device needs:
 
   * PPoly knots [1000] and coefficients [999][2][4] (FP64)      -> Path.__call__, get_direction
   * polyline vertices [n][2] and chord-length prefix sums [n]     -> LineString.project
-  * one (chord, deviation) capsule per 32 consecutive segments    -> two-level exact search
+  * one (chord, deviation) capsule per 8, 32 and 512 consecutive segments -> exact hierarchical search
   * length, end point, origin
 
 Construction stays on the host with SciPy (the reference does the same); only
@@ -25,6 +25,7 @@ from scipy import interpolate
 
 PATH_BLOCK = int(os.environ.get("AUV_PATH_BLOCK", 32))  # must equal AUV_PATH_BLOCK in include/auv_b200.h (env override: tuning builds only)
 PATH_SUPER = int(os.environ.get("AUV_PATH_SUPER", 16))  # blocks per superblock, AUV_PATH_SUPER (env override: tuning builds only)
+PATH_SUB = 8  # segments per sub-block, AUV_PATH_SUB
 N_KNOTS = 1000
 PP_W = 12  # AUV_PP_W
 HDR_DTYPE = np.dtype([("v0", "<i4"), ("nseg", "<i4"), ("b0", "<i4"), ("s0", "<i4"), ("ox", "<f8"), ("oy", "<f8"),
@@ -43,6 +44,8 @@ class PathTable:
     blk_dev: np.ndarray  # [nblk, 2] float32 (1/|e|^2, deviation)
     sb_chord: np.ndarray  # [nsb, 4] float32
     sb_dev: np.ndarray  # [nsb, 2] float32
+    sub_chord: np.ndarray  # [ceil(nseg / 8), 4] float32
+    sub_dev: np.ndarray  # [ceil(nseg / 8), 2] float32
     origin: np.ndarray  # [2]
     length: float
     end: np.ndarray  # [2]
@@ -115,6 +118,7 @@ def build_path(waypoints) -> PathTable:
     rel = poly - origin
     blk_chord, blk_dev = _capsules(rel, nseg, PATH_BLOCK)
     sb_chord, sb_dev = _capsules(rel, nseg, PATH_BLOCK * PATH_SUPER)
+    sub_chord, sub_dev = _capsules(rel, nseg, PATH_SUB)
     return PathTable(
         knots=np.ascontiguousarray(spline.x),
         coef=coef,
@@ -124,6 +128,8 @@ def build_path(waypoints) -> PathTable:
         blk_dev=blk_dev,
         sb_chord=sb_chord,
         sb_dev=sb_dev,
+        sub_chord=sub_chord,
+        sub_dev=sub_dev,
         origin=origin,
         length=length,
         end=np.array(spline(length), dtype=np.float64),
@@ -134,7 +140,9 @@ def build_path(waypoints) -> PathTable:
 class PathBank:
     """A list of PathTable concatenated into the flat arrays of ``AuvPathBank``: one 64 B header
     per path, capsule tables whose per-path offsets are even (so a CTA can bulk-copy a path's
-    tables into shared memory in 16 B units), one 96 B record per PCHIP piece."""
+    tables into shared memory in 16 B units), one 96 B record per PCHIP piece.  A path's sub-block
+    table is padded to PATH_BLOCK // PATH_SUB entries per (padded) block, so it starts at that multiple
+    of the path's first block."""
 
     def __init__(self, tables: Sequence[PathTable]):
         if len(tables) == 0:
@@ -150,18 +158,22 @@ class PathBank:
             self.blk_off[i + 1] = self.blk_off[i] + even(len(t.blk_dev))
             self.sb_off[i + 1] = self.sb_off[i] + even(len(t.sb_dev))
 
-        def padded(parts, width):
-            out = np.zeros((int(sum(even(len(p)) for p in parts)), width), dtype=np.float32)
+        def padded(parts, width, slot=lambda p: even(len(p))):
+            out = np.zeros((int(sum(slot(p) for p in parts)), width), dtype=np.float32)
             o = 0
             for p in parts:
                 out[o:o + len(p)] = p
-                o += even(len(p))
+                o += slot(p)
             return out
+
+        per_blk = PATH_BLOCK // PATH_SUB
 
         self.sb_chord = padded([t.sb_chord for t in tables], 4)
         self.sb_dev = padded([t.sb_dev for t in tables], 2)
         self.blk_chord = padded([t.blk_chord for t in tables], 4)
         self.blk_dev = padded([t.blk_dev for t in tables], 2)
+        self.sub_chord = padded([t.sub_chord for t in tables], 4, slot=lambda p: per_blk * even((len(p) + per_blk - 1) // per_blk))
+        self.sub_dev = padded([t.sub_dev for t in tables], 2, slot=lambda p: per_blk * even((len(p) + per_blk - 1) // per_blk))
         self.poly_xy = np.concatenate([t.poly for t in tables], axis=0)
         self.poly_cum = np.concatenate([t.cum for t in tables])
         self.origin = np.stack([t.origin for t in tables])
@@ -217,6 +229,8 @@ class PathBank:
             sb_chord=dev(self.sb_chord, torch.float32),
             sb_dev=dev(self.sb_dev, torch.float32),
             pp=dev(self.piece_array(), torch.float64),
+            sub_chord=dev(self.sub_chord, torch.float32),
+            sub_dev=dev(self.sub_dev, torch.float32),
         )
 
 
@@ -230,7 +244,9 @@ class DevicePathBank:
     ``vcap``: a PCHIP curve is monotone per coordinate between its knots, so its length is at most the L1
     length of the waypoint polygon; for ``RandomCurveThroughOrigin(length=800)`` with up to 5 waypoints
     (movingobstacles.py:30-31) that is < 4.08 x 800 m = 3264 m -> 32642 vertices: the default never overflows
-    for that family (paths of ~1.7 km do occur among a few thousand samples)."""
+    for that family (paths of ~1.7 km do occur among a few thousand samples).  It is rounded up to a multiple of
+    2 x PATH_BLOCK x PATH_SUPER, so that every slot's first block and superblock are even (the step bulk-copies
+    these tables in 16 B units)."""
 
     n_knots = N_KNOTS
 
@@ -242,7 +258,7 @@ class DevicePathBank:
             if w.ndim != 2 or w.shape[0] != 2 or not (2 <= w.shape[1] <= 8):
                 raise ValueError(f"device-built paths take 2..8 waypoints of shape [2, n], got {w.shape}")
         self.n_paths = len(self.waypoints)
-        span = PATH_BLOCK * PATH_SUPER
+        span = 2 * PATH_BLOCK * PATH_SUPER
         self.vcap = (int(vcap) + span - 1) // span * span
         self._tables = None
         self._dev = None
@@ -273,6 +289,7 @@ class DevicePathBank:
             blk_dev=z((P * V // PATH_BLOCK, 2), torch.float32),
             sb_chord=z((P * V // (PATH_BLOCK * PATH_SUPER), 4), torch.float32),
             sb_dev=z((P * V // (PATH_BLOCK * PATH_SUPER), 2), torch.float32), pp=z((P, N_KNOTS - 1, PP_W), torch.float64),
+            sub_chord=z((P * V // PATH_SUB, 4), torch.float32), sub_dev=z((P * V // PATH_SUB, 2), torch.float32),
         )
 
     def build_struct(self, arrays):
@@ -281,7 +298,8 @@ class DevicePathBank:
         a = arrays
         return _lib.AuvPathBuild(a["hdr"].data_ptr(), a["poly_xy"].data_ptr(), a["poly_cum"].data_ptr(), a["poly_f32"].data_ptr(),
                                  a["blk_chord"].data_ptr(), a["blk_dev"].data_ptr(), a["sb_chord"].data_ptr(),
-                                 a["sb_dev"].data_ptr(), a["pp"].data_ptr(), N_KNOTS, self.vcap)
+                                 a["sb_dev"].data_ptr(), a["pp"].data_ptr(), N_KNOTS, self.vcap, a["sub_chord"].data_ptr(),
+                                 a["sub_dev"].data_ptr())
 
     def device_arrays(self, device):
         """Allocate the slots and build every path on the device."""

@@ -191,7 +191,7 @@ class AUVVecEnv:
         self.paths = _lib.AuvPathBank(
             bank.n_paths, getattr(bank, "n_knots", None) or bank.knots.shape[1], b["hdr"].data_ptr(), b["poly_xy"].data_ptr(), b["poly_cum"].data_ptr(),
             b["poly_f32"].data_ptr(), b["blk_chord"].data_ptr(), b["blk_dev"].data_ptr(), b["sb_chord"].data_ptr(), b["sb_dev"].data_ptr(),
-            b["pp"].data_ptr(),
+            b["pp"].data_ptr(), b["sub_chord"].data_ptr(), b["sub_dev"].data_ptr(),
         )
 
         # ---- scenario pool

@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define AUV_ABI_VERSION 19
+#define AUV_ABI_VERSION 20
 
 #define AUV_EINVAL (-1)  /* bad argument / NULL pointer / unsupported size */
 #define AUV_ENOTSUP (-2) /* feature not built */
@@ -67,6 +67,7 @@ extern "C" {
 #ifndef AUV_PATH_SUPER
 #define AUV_PATH_SUPER 16     /* blocks per projection superblock (8 / 16 / 32 swept: profiles/r1j_variants.txt) */
 #endif
+#define AUV_PATH_SUB 8        /* polyline segments per sub-block (a block holds AUV_PATH_BLOCK / AUV_PATH_SUB of them) */
 #define AUV_NAV_W 24          /* doubles per env in AuvBatch.nav */
 #define AUV_REC_BYTES 80      /* bytes per obstacle record in AuvBatch.rec */
 #define AUV_MAX_POLY_VERTS 192 /* vertices of one world polygon incl. the closing one */
@@ -129,7 +130,8 @@ typedef struct AuvPathHdr {
   int32_t v0;      /* first polyline vertex in poly_xy / poly_cum                          */
   int32_t nseg;    /* polyline segments (vertices - 1); blocks = ceil(nseg / AUV_PATH_BLOCK),
                       superblocks = ceil(blocks / AUV_PATH_SUPER)                           */
-  int32_t b0;      /* first block capsule (even, so the tables can be bulk-copied)          */
+  int32_t b0;      /* first block capsule (even, so the tables can be bulk-copied); the path's
+                      sub-block capsules start at (AUV_PATH_BLOCK / AUV_PATH_SUB) * b0       */
   int32_t s0;      /* first superblock capsule (even)                                       */
   double ox, oy;   /* origin the FP32 capsules are relative to                              */
   double length;   /* Path.length                                                           */
@@ -155,6 +157,12 @@ typedef struct AuvPathBank {
   const double* pp;        /* [n_paths][n_knots-1][AUV_PP_W]: knot j, knot j+1, x: c0..c3,
                               y: c0..c3 (value = ((c0 t + c1) t + c2) t + c3, t = s - knot j),
                               2 unused                                                   */
+  const float* sub_chord;  /* [total_blocks * AUV_PATH_BLOCK / AUV_PATH_SUB][4] capsules of AUV_PATH_SUB
+                              segments, same layout as blk_chord; a path's table has
+                              (AUV_PATH_BLOCK / AUV_PATH_SUB) x its block count entries.  Optional:
+                              NULL (with sub_dev) only costs speed, the refine then evaluates
+                              every segment of a candidate block                          */
+  const float* sub_dev;    /* [total_blocks * AUV_PATH_BLOCK / AUV_PATH_SUB][2] same layout as blk_dev */
 } AuvPathBank;
 
 /* Scenario pool: the read-only part of what a scenario plug-in's _generate() produces
@@ -486,7 +494,9 @@ int auv_refresh_finished(const AuvConfig* cfg, const AuvRayTable* rays, const Au
  * plus the tables of AuvPathBank (PPoly piece records, chord-length prefix sums, FP32 polyline,
  * block / superblock capsules, header), one CTA per path, SciPy's / NumPy's evaluation order with
  * explicit round-to-nearest operations.  Slot layout: path p owns vertices [p vcap, (p + 1) vcap),
- * blocks [p vcap / 32, ...), superblocks [p vcap / 512, ...); vcap a multiple of 512.  A polyline that
+ * blocks [p vcap / 32, ...), sub-blocks [p vcap / 8, ...), superblocks [p vcap / 512, ...); vcap a multiple
+ * of 1024 (so that every path's first block and superblock are even).  sub_chord / sub_dev may be NULL
+ * (then they are not built; see AuvPathBank).  A polyline that
  * does not fit raises AUV_STATUS_PATH_TOO_LONG.  waypoints: device [n][2][8] (x row, y row; as passed to
  * the reference's Path()), n_wp: device [n] (2..8), path_ids: device [n] slots to write, NULL = 0..n-1. */
 typedef struct AuvPathBuild {
@@ -501,6 +511,8 @@ typedef struct AuvPathBuild {
   double* pp;
   int32_t n_knots; /* 1000 */
   int32_t vcap;
+  float* sub_chord;
+  float* sub_dev;
 } AuvPathBuild;
 int auv_pathbank_build(const double* waypoints, const int32_t* n_wp, const int32_t* path_ids, int n,
                        const AuvPathBuild* out, int32_t* status, void* stream);
