@@ -332,6 +332,11 @@ __device__ AUV_PROJECT_INLINE double project_group(const AuvPathBank& pb, const 
       best_seg = oi;
     }
   }
+  // a bound that pruned every segment would leave best_seg = 0x7fffffff: flag it, and keep the debug build's read in bounds
+  AUV_CHECK(status, best_seg >= 0 && best_seg < nseg);
+#ifdef AUV_DEBUG_BOUNDS
+  best_seg = min(max(best_seg, 0), nseg - 1);
+#endif
   seg_out = best_seg;
   // segmentNearestMeasure of the winning segment
   const double2 A = poly[best_seg], B = poly[best_seg + 1];

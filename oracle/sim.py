@@ -241,6 +241,24 @@ def cast_ray(angle, p0, sensor_range, obstacles, with_obstacle=False):
     return (d, who) if with_obstacle else d
 
 
+def cast_ray_runner_up(angle, p0, sensor_range, obstacles):
+    """cast_ray(with_obstacle=True) plus the nearest intersection on any OTHER obstacle: the margin by which
+    the nearest obstacle -- whose velocity the ray reports -- wins.  Returns (d, obstacle, d_other,
+    other_obstacle); (sensor_range, None, inf, None) for a clear ray, (d, obstacle, inf, None) for one hit."""
+    p1 = (p0[0] + math.cos(angle) * sensor_range, p0[1] + math.sin(angle) * sensor_range)
+    hits = []
+    for i, ob in enumerate(obstacles):
+        d = 0.0 if ob.filled and G.point_in_ring(p0, ob.ring) else G.ray_ring_min_distance_np(p0, p1, ob.ring)
+        if d is not None:
+            hits.append((d, i, ob))
+    if not hits:
+        return sensor_range, None, math.inf, None
+    hits.sort(key=lambda h: (h[0], h[1]))  # first obstacle on ties, as cast_ray
+    d, _, who = hits[0]
+    d2, _, who2 = next((h for h in hits[1:] if h[2] is not who), (math.inf, -1, None))
+    return d, who, d2, who2
+
+
 def relative_speed(angle, ob):
     """sensor.py:118-128: Rz(-sensor_angle - pi/2) applied to the obstacle's last displacement (dx, dy)."""
     if ob is None or ob.static:

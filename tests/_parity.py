@@ -32,8 +32,9 @@ def oracle_cfg(config, **extra):
     return d
 
 
-def rollout_oracle(scn, config, actions, test_mode=True, **cfg_extra):
-    """actions: [T, M, 2].  Returns dict of arrays [T(+1), M, ...] (stops an env at done)."""
+def rollout_oracle(scn, config, actions, test_mode=True, on_step=None, **cfg_extra):
+    """actions: [T, M, 2].  Returns dict of arrays [T(+1), M, ...] (stops an env at done).
+    on_step(t, m, env), if given, is called after every step with the stepped OracleEnv."""
     from oracle.sim import OracleEnv
 
     T, M = actions.shape[0], scn.n_scenarios
@@ -76,6 +77,8 @@ def rollout_oracle(scn, config, actions, test_mode=True, **cfg_extra):
                 out["windows"][t][m] = {slot[id(o)]: w for o, w in zip(env.vessel.nearby, env.vessel.windows)}
             else:
                 out["windows"][t][m] = {}
+            if on_step is not None:
+                on_step(t, m, env)
             if done:
                 break
         out["n_tests"][m] = env.vessel.n_tests
@@ -270,11 +273,11 @@ def live_sample_compare(env, config, acts, horizon, n_sample, start, prefer_reco
             rep["range_max_abs"] = max(rep["range_max_abs"], float(derr.max()))
             rep["obs_max_abs"] = max(rep["obs_max_abs"], float(oerr))
             rep["reward_max_abs"] = max(rep["reward_max_abs"], rerr)
-            if done:  # VecEnv auto-reset: the env moves on to pool scenario (m + N) mod M
+            if done:  # VecEnv auto-reset: the env moves on to pool scenario (m + stride) mod M
                 from oracle.sim import OracleEnv
 
                 rep["resets"] += 1
-                m = (m + N) % M
+                m = (m + (env.reset_stride or N)) % M  # a ring group strides by the whole ring, not its own size
                 o = OracleEnv(scn_host.describe(m), oracle_cfg(config, **cfg_extra), test_mode=False)
                 first = o.reset()  # (the constructor already reset once; the second reset is identical)
                 ferr = np.abs(g["obs"][k] - first).max()
