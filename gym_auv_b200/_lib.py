@@ -8,7 +8,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("AUV_B200_LIB", os.path.join(_HERE, "libauv_b200.so"))  # override: tuning builds only
-ABI_VERSION = 20
+ABI_VERSION = 21
 REC_BYTES = 80
 MAX_POLY_VERTS = 192
 STATUS_REC_OVERFLOW = 1
@@ -16,6 +16,7 @@ STATUS_GEN_GAVE_UP = 2
 STATUS_POLY_TOO_LARGE = 4
 STATUS_PATH_TOO_LONG = 8
 STATUS_BOUNDS = 16
+STATUS_GEN_LAND_BLOCKED = 32
 PP_W = 12
 PATH_STAGE_BLOCKS = 512
 NAV_W = 24
@@ -211,6 +212,7 @@ class AuvGenParams(C.Structure):
         ("st_radius_mean", C.c_double),
         ("path_group", C.c_int32),
         ("path_period", C.c_int32),
+        ("land_clearance", C.c_double),
     ]
 
 

@@ -1,7 +1,9 @@
 // auv_generate.cuh -- GPU-side scenario generation for the MovingObstacles family:
 // what MovingObstacles._generate (envs/movingobstacles.py:28-95) and helpers.generate_obstacle
-// (utils/helpers.py:5-35) sample per episode, batched, one thread per (scenario, obstacle slot),
-// counter-based Philox4x32-10 streams (SURVEY.md section 8f rank 1).  The reference mixes a
+// (utils/helpers.py:5-35) sample per episode, batched in two launches -- one thread per scenario for the
+// path and vessel start, then one per (scenario, obstacle slot) --, counter-based Philox4x32-10 streams
+// (SURVEY.md section 8f rank 1).  In a pool with a shared land-polygon world every placed object must also
+// be clear of land (land_clear below; DESIGN.md section 6b); without a world the draws are unchanged.  The reference mixes a
 // seeded RandomState with the global unseeded np.random (SURVEY quirk B10), so its streams
 // cannot be reproduced; parity here is distributional + the acceptance rule, and every
 // generated scenario can be pulled back to the host and replayed through the oracle.
@@ -62,6 +64,7 @@ struct GenRng {
 #define AUV_GEN_SLOT_VESSEL 0xFFFFu
 #define AUV_GEN_SLOT_PATH 0xFFFEu
 #define AUV_GEN_MAX_TRIES 100000
+#define AUV_GEN_VESSEL_TRIES 4096  // vessel-start draws before AUV_STATUS_GEN_LAND_BLOCKED
 
 __device__ __forceinline__ void gen_path_point(const AuvPathBank& pb, int pid, double L, double s, double& x, double& y,
                                                double& dir) {
@@ -72,44 +75,137 @@ __device__ __forceinline__ void gen_path_point(const AuvPathBank& pb, int pid, d
   dir = atan2(a.dy, a.dx);  // Path.get_direction, path.py:72-82
 }
 
-// thread per (listed scenario, slot): slots [0, Km) moving, [Km, Km+Ks) static, slot Km+Ks writes the
-// per-scenario fields.  ids == nullptr: scenarios [0, n_ids).
-__global__ void __launch_bounds__(128) k_generate_moving_obstacles(const __grid_constant__ AuvGenParams gp,
-                                                                    const __grid_constant__ AuvPathBank pb,
-                                                                    const __grid_constant__ AuvScenarioPool pool,
-                                                                    const int* __restrict__ ids, int n_ids,
-                                                                    const int* __restrict__ n_ids_dev,
-                                                                    int* __restrict__ status) {
-  const int km = pool.k_moving, ks = pool.k_static, per = km + ks + 1;
-  const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (n_ids_dev != nullptr) n_ids = min(n_ids, *n_ids_dev);  // list length decided on the device (auv_refresh_finished)
-  if (gid >= (long long)n_ids * per) return;
-  const int li = (int)(gid / per), slot = (int)(gid - (long long)li * per);
+// ---- "clear of land by d": (px, py) is outside every world polygon (even-odd rule on the closed ring) and its
+// FP64 distance to every ring is > d.  Not world_polygon_distance: that is the step's FP32 culling test.
+// Polygon j alone; the ring is read from global memory, so any perimeter length is accepted.  The crossing and
+// distance tests are written without divisions (the division slow path is a call, which makes the
+// rejection loops spill); they decide as oracle.geos_lite.point_in_ring / point_ring_distance do up to rounding.
+__device__ __forceinline__ bool land_polygon_clear(const AuvScenarioPool& pool, int j, double px, double py, double d) {
+  const double cx = pool.world_circle[3 * j], cy = pool.world_circle[3 * j + 1], rr = pool.world_circle[3 * j + 2] + d;
+  if ((px - cx) * (px - cx) + (py - cy) * (py - cy) > rr * rr) return true;  // enclosing circle out of reach
+  const double2* v = reinterpret_cast<const double2*>(pool.world_verts);
+  const int k1 = pool.world_voff[j + 1];
+  const double d2 = d * d;
+  bool inside = false;
+  double2 a = v[pool.world_voff[j]];
+  for (int k = pool.world_voff[j] + 1; k < k1; ++k) {
+    const double2 b = v[k];
+    const double ex = b.x - a.x, ey = b.y - a.y, qx = a.x - px, qy = a.y - py;
+    const double cr = qx * ey - qy * ex;  // (a - p) x (b - a): its sign tells on which side of the edge p lies
+    if ((a.y > py) != (b.y > py)) {  // crossing number: the edge crosses the horizontal through p ...
+      if (cr == 0.0) return false;   // ... at p itself (on the boundary = inside)
+      if ((cr > 0.0) == (ey > 0.0)) inside = !inside;  // ... right of p
+    }
+    // point-segment distance (GEOS Distance::pointToSegment), squared and compared with d^2
+    const double len2 = ex * ex + ey * ey, t = -(qx * ex + qy * ey);  // t = (p - a).(b - a)
+    double dist2;
+    if (t <= 0.0 || len2 == 0.0) {
+      dist2 = qx * qx + qy * qy;
+    } else if (t >= len2) {
+      dist2 = (b.x - px) * (b.x - px) + (b.y - py) * (b.y - py);
+    } else {
+      dist2 = -1.0;  // interior foot: |cr|^2 / len2 <= d^2
+      if (cr * cr <= d2 * len2) return false;
+    }
+    if (dist2 >= 0.0 && dist2 <= d2) return false;  // early exit: within d of this edge
+    a = b;
+  }
+  return !inside;
+}
+
+// the whole world: the cells of the pool's uniform grid that the disc of radius d overlaps (cell ranges computed
+// as World.grid computes a circle's), or every polygon when the pool has no grid
+__device__ __forceinline__ bool land_clear(const AuvScenarioPool& pool, double px, double py, double d) {
+  if (pool.n_world <= 0) return true;
+  if (pool.world_cell_off == nullptr) {
+    for (int j = 0; j < pool.n_world; ++j)
+      if (!land_polygon_clear(pool, j, px, py, d)) return false;
+    return true;
+  }
+  const double cell = pool.world_grid_cell;
+  const double fx0 = floor((px - d - pool.world_grid_x0) / cell), fx1 = floor((px + d - pool.world_grid_x0) / cell);
+  const double fy0 = floor((py - d - pool.world_grid_y0) / cell), fy1 = floor((py + d - pool.world_grid_y0) / cell);
+  const int nx = pool.world_grid_nx, ny = pool.world_grid_ny;
+  if (!(fx1 >= 0.0 && fy1 >= 0.0 && fx0 <= (double)(nx - 1) && fy0 <= (double)(ny - 1))) return true;  // off the grid
+  const int ix0 = (int)fmax(fx0, 0.0), ix1 = (int)fmin(fx1, (double)(nx - 1));
+  const int iy0 = (int)fmax(fy0, 0.0), iy1 = (int)fmin(fy1, (double)(ny - 1));
+  for (int iy = iy0; iy <= iy1; ++iy)
+    for (int ix = ix0; ix <= ix1; ++ix) {
+      const int c = iy * nx + ix;
+      for (int it = pool.world_cell_off[c]; it < pool.world_cell_off[c + 1]; ++it)
+        if (!land_polygon_clear(pool, pool.world_cell_items[it], px, py, d)) return false;
+    }
+  return true;
+}
+
+// Both generator kernels are launched with 128 threads.  __maxnreg__ instead of __launch_bounds__(128): with the
+// latter ptxas kept the rejection loops at 48-64 registers and spilled what lives across the calls of the
+// FP64 division / trig slow paths.
+// Launch 1 of 2, thread per listed scenario: path choice and the vessel start, written to pool.path_id /
+// vessel_init.  ids == nullptr: scenarios [0, n_ids); n_ids_dev: list length decided on the device
+// (auv_refresh_finished).
+__global__ void __maxnreg__(128) k_generate_scenario_heads(const __grid_constant__ AuvGenParams gp,
+                                                                  const __grid_constant__ AuvPathBank pb,
+                                                                  const __grid_constant__ AuvScenarioPool pool,
+                                                                  const int* __restrict__ ids, int n_ids,
+                                                                  const int* __restrict__ n_ids_dev,
+                                                                  int* __restrict__ status) {
+  asm volatile("griddepcontrol.launch_dependents;");  // let k_generate_moving_obstacles be dispatched now
+  if (n_ids_dev != nullptr) n_ids = min(n_ids, *n_ids_dev);
+  const int li = blockIdx.x * blockDim.x + threadIdx.x;
+  if (li >= n_ids) return;
   const int m = ids ? ids[li] : li;
-  // ---- per-scenario draws, recomputed by every thread of the scenario (same stream => same values)
   GenRng rp(gp.seed, (unsigned)m, AUV_GEN_SLOT_PATH, gp.epoch);
   // path choice: uniform over the bank (movingobstacles.py:28-31 draws a fresh curve), or -- path-major
   // pools -- the path the slot is laid out for: consecutive groups of path_group scenarios share a path
   const double upath = rp.u01();
   const int pid = gp.path_group > 0 ? (int)(((long long)m % gp.path_period) / gp.path_group) % pb.n_paths
                                     : min(pb.n_paths - 1, (int)(upath * pb.n_paths));
-  const double L = pb.hdr[pid].length;
   GenRng rv(gp.seed, (unsigned)m, AUV_GEN_SLOT_VESSEL, gp.epoch);
   double x0, y0, dir0;
-  gen_path_point(pb, pid, L, 0.0, x0, y0, dir0);
-  // movingobstacles.py:34-38: init_state = path(0) + 50 (rand(2) - 0.5); angle = dir(0) + 2 pi (rand - 0.5)
-  const double vx = x0 + gp.init_pos_jitter * (rv.u01() - 0.5);
-  const double vy = y0 + gp.init_pos_jitter * (rv.u01() - 0.5);
-  const double vpsi = princip(dir0 + 2.0 * AUV_PI * (rv.u01() - 0.5));
-  double* wv = const_cast<double*>(pool.vessel_init);
-  if (slot == km + ks) {
-    const_cast<int*>(pool.path_id)[m] = pid;
-    wv[3ll * m + 0] = vx;
-    wv[3ll * m + 1] = vy;
-    wv[3ll * m + 2] = vpsi;
-    return;
+  gen_path_point(pb, pid, pb.hdr[pid].length, 0.0, x0, y0, dir0);
+  // movingobstacles.py:34-38: init_state = path(0) + 50 (rand(2) - 0.5); angle = dir(0) + 2 pi (rand - 0.5);
+  // in a world the start must be clear of land by land_clearance: redraw from the same stream
+  double vx, vy, vpsi;
+  for (int tries = 1;; ++tries) {
+    vx = x0 + gp.init_pos_jitter * (rv.u01() - 0.5);
+    vy = y0 + gp.init_pos_jitter * (rv.u01() - 0.5);
+    vpsi = princip(dir0 + 2.0 * AUV_PI * (rv.u01() - 0.5));
+    if (land_clear(pool, vx, vy, gp.land_clearance)) break;
+    if (tries >= AUV_GEN_VESSEL_TRIES) {  // keep the last draw
+      if (status) atomicOr(status, AUV_STATUS_GEN_LAND_BLOCKED);
+      break;
+    }
   }
-  // ---- helpers.generate_obstacle: rejection until clear of the vessel and of the goal
+  const_cast<int*>(pool.path_id)[m] = pid;
+  double* wv = const_cast<double*>(pool.vessel_init);
+  wv[3ll * m + 0] = vx;
+  wv[3ll * m + 1] = vy;
+  wv[3ll * m + 2] = vpsi;
+}
+
+// Launch 2 of 2, thread per (listed scenario, obstacle slot): slots [0, Km) moving, [Km, Km+Ks) static; the
+// path and vessel start are read back from what k_generate_scenario_heads wrote.
+__global__ void __maxnreg__(128) k_generate_moving_obstacles(const __grid_constant__ AuvGenParams gp,
+                                                                    const __grid_constant__ AuvPathBank pb,
+                                                                    const __grid_constant__ AuvScenarioPool pool,
+                                                                    const int* __restrict__ ids, int n_ids,
+                                                                    const int* __restrict__ n_ids_dev,
+                                                                    int* __restrict__ status) {
+  // launched as a programmatic dependent of k_generate_scenario_heads: wait until it has completed and its
+  // writes are visible (a no-op after an ordinary launch)
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  const int km = pool.k_moving, ks = pool.k_static, per = km + ks;
+  const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (n_ids_dev != nullptr) n_ids = min(n_ids, *n_ids_dev);
+  if (gid >= (long long)n_ids * per) return;
+  const int li = (int)(gid / per), slot = (int)(gid - (long long)li * per);
+  const int m = ids ? ids[li] : li;
+  const int pid = pool.path_id[m];
+  const double L = pb.hdr[pid].length;
+  const double vx = pool.vessel_init[3ll * m], vy = pool.vessel_init[3ll * m + 1];
+  // ---- helpers.generate_obstacle: rejection until clear of the vessel and of the goal (and, in a world, the
+  // centre / track start clear of land by the radius / width)
   const bool moving = slot < km;
   const double disp_std = moving ? gp.mov_disp_std : gp.st_disp_std;
   const double mean = moving ? gp.mov_width_mean : gp.st_radius_mean;
@@ -131,7 +227,7 @@ __global__ void __launch_bounds__(128) k_generate_moving_obstacles(const __grid_
     rad = fmax(1.0, (double)r.poisson(mean));
     const double dv = sqrt((ox - vx) * (ox - vx) + (oy - vy) * (oy - vy)) - gp.vessel_width - rad;
     const double dg = sqrt((ox - gx) * (ox - gx) + (oy - gy) * (oy - gy)) - rad;
-    if (fmin(dv, dg) > 0.0) break;
+    if (fmin(dv, dg) > 0.0 && land_clear(pool, ox, oy, rad)) break;
     if (tries >= AUV_GEN_MAX_TRIES) {
       if (status) atomicOr(status, AUV_STATUS_GEN_GAVE_UP);
       break;

@@ -2276,6 +2276,41 @@ int auv_step_host(const AuvConfig* cfg, const AuvRayTable* rays, const AuvPathBa
   return cuda_check(cudaStreamSynchronize(s), "sync");
 }
 
+static int check_gen_world(const AuvGenParams* gp, const AuvScenarioPool* pool) {
+  if (pool->n_world < 0) return set_err(AUV_EINVAL, "n_world < 0");
+  if (pool->n_world == 0) return 0;
+  if (!pool->world_circle || !pool->world_voff || !pool->world_verts) return set_err(AUV_EINVAL, "world arrays are NULL");
+  if (pool->world_cell_off &&
+      (!pool->world_cell_items || pool->world_grid_nx <= 0 || pool->world_grid_ny <= 0 || !(pool->world_grid_cell > 0.0)))
+    return set_err(AUV_EINVAL, "world grid: NULL items or empty grid");
+  if (!(gp->land_clearance >= 0.0)) return set_err(AUV_EINVAL, "land_clearance must be >= 0");
+  return 0;
+}
+
+// both launches of the generator (auv_generate.cuh): per scenario, then per (scenario, obstacle slot)
+static int launch_generate(const AuvGenParams* gp, const AuvPathBank* paths, const AuvScenarioPool* pool,
+                           const int32_t* ids, int n_ids, const int32_t* n_ids_dev, int32_t* status, cudaStream_t s) {
+  const int threads = 128;
+  auv::k_generate_scenario_heads<<<(unsigned)((n_ids + threads - 1) / threads), threads, 0, s>>>(*gp, *paths, *pool, ids, n_ids,
+                                                                                               n_ids_dev, status);
+  if (int rc = cuda_check(cudaGetLastError(), "k_generate_scenario_heads")) return rc;
+  const long long total = (long long)n_ids * (pool->k_moving + pool->k_static);
+  if (total == 0) return 0;
+  // programmatic dependent launch: the slot grid is dispatched while the per-scenario grid runs and waits for
+  // its results on the device (griddepcontrol.wait), so the split costs no launch gap
+  cudaLaunchConfig_t lc = {};
+  lc.gridDim = dim3((unsigned)((total + threads - 1) / threads));
+  lc.blockDim = dim3(threads);
+  lc.stream = s;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  lc.attrs = at;
+  lc.numAttrs = 1;
+  return cuda_check(cudaLaunchKernelEx(&lc, auv::k_generate_moving_obstacles, *gp, *paths, *pool, ids, n_ids, n_ids_dev, status),
+                    "k_generate_moving_obstacles");
+}
+
 int auv_generate_moving_obstacles(const AuvGenParams* gp, const AuvPathBank* paths, const AuvScenarioPool* pool,
                                   const int32_t* ids, int n_ids, int32_t* status, void* stream) {
   if (!gp || !paths || !pool) return set_err(AUV_EINVAL, "NULL argument");
@@ -2287,12 +2322,8 @@ int auv_generate_moving_obstacles(const AuvGenParams* gp, const AuvPathBank* pat
                              !pool->mov_pos0 || !pool->mov_disp0 || !pool->mov_counter0))
     return set_err(AUV_EINVAL, "moving-obstacle arrays are NULL");
   if (pool->k_static > 0 && (!pool->st_pos || !pool->st_radius)) return set_err(AUV_EINVAL, "static-obstacle arrays are NULL");
-  const long long total = (long long)n_ids * (pool->k_moving + pool->k_static + 1);
-  const int threads = 128;
-  const long long blocks = (total + threads - 1) / threads;
-  auv::k_generate_moving_obstacles<<<(unsigned)blocks, threads, 0, (cudaStream_t)stream>>>(*gp, *paths, *pool, ids, n_ids,
-                                                                                          nullptr, status);
-  return cuda_check(cudaGetLastError(), "k_generate_moving_obstacles");
+  if (int rc = check_gen_world(gp, pool)) return rc;
+  return launch_generate(gp, paths, pool, ids, n_ids, nullptr, status, (cudaStream_t)stream);
 }
 
 int auv_linear_wrap(double dt, double counter0, int vel_len, int32_t* first_wrap, int32_t* wrap_period) {
@@ -2386,17 +2417,14 @@ int auv_refresh_finished(const AuvConfig* cfg, const AuvRayTable* rays, const Au
     return set_err(AUV_EINVAL, "refresh scratch: NULL array or capacity not in 1..worker.n_envs");
   if (pool->n_scenarios != 2 * (live->reset_stride > 0 ? live->reset_stride : live->n_envs))
     return set_err(AUV_EINVAL, "refresh needs a pool of exactly 2 * reset_stride (default n_envs) scenarios");
-  if (pool->n_world > 0) return set_err(AUV_ENOTSUP, "scenario generation with a shared land-polygon world");
+  if (int rc = check_gen_world(gp, pool)) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   const int threads = 128;
   if (int rc = cuda_check(cudaMemsetAsync(rs->count, 0, sizeof(int32_t), s), "memset")) return rc;
   auv::k_refresh_collect<<<(live->n_envs + threads - 1) / threads, threads, 0, s>>>(*live, pool->n_scenarios, rs->seen_episode,
                                                                                     rs->ids, rs->count, rs->capacity);
   if (int rc = cuda_check(cudaGetLastError(), "k_refresh_collect")) return rc;
-  const long long total = (long long)rs->capacity * (pool->k_moving + pool->k_static + 1);
-  auv::k_generate_moving_obstacles<<<(unsigned)((total + threads - 1) / threads), threads, 0, s>>>(
-      *gp, *paths, *pool, rs->ids, rs->capacity, rs->count, live->status);
-  if (int rc = cuda_check(cudaGetLastError(), "k_generate_moving_obstacles")) return rc;
+  if (int rc = launch_generate(gp, paths, pool, rs->ids, rs->capacity, rs->count, live->status, s)) return rc;
   return reset_cache_fill(cfg, rays, paths, pool, worker, worker_out, rs->ids, 0, rs->capacity, rs->count, stream);
 }
 

@@ -21,6 +21,9 @@ import numpy as np
 from .pathbank import DevicePathBank, PathBank, PathTable, build_path, random_curve_waypoints
 
 VESSEL_TRACK_LEN = 9999  # a 10000-point trajectory yields 9999 per-second velocities
+# GPU scenario generation in a shared land-polygon world: a vessel start must be clear of land by this much
+# (outside every polygon, farther from every ring) -- the margin random_land keeps around vessel starts
+LAND_CLEARANCE = 30.0
 
 
 def princip(a):
@@ -527,6 +530,24 @@ def land_scenarios(n_scenarios: int, n_polygons: int = 512, n_moving: int = 0, n
 
     scn = moving_obstacles(n_scenarios, n_moving, n_static, seed=seed, n_paths=n_paths, name="LandPolygons")
     scn.world_polygons = random_land(n_polygons, extent, seed=seed + 77, keep_clear=scn.vessel_init[:, :2])
+    return scn
+
+
+def land_template(n_scenarios: int, n_polygons: int = 512, n_moving: int = 16, n_static: int = 16, seed: int = 0,
+                  n_paths: int = 1024, extent: float = 6000.0, path_period: Optional[int] = None,
+                  device_paths: bool = False) -> ScenarioSet:
+    """``moving_obstacles_template`` inside a shared world of ``random_land`` polygons: the input of
+    ``AUVVecEnv.regenerate_scenarios`` for the BASELINE config 4 shape with a fresh scenario per episode.
+    Land is kept clear of every bank path's first and last waypoint by ``25 sqrt(2) + LAND_CLEARANCE + 1`` m,
+    so that every corner of a path's +-25 m start square is clear of land by LAND_CLEARANCE and the
+    template's own bank never forces a vessel start to be redrawn."""
+    from .polygons import random_land
+
+    scn = moving_obstacles_template(n_scenarios, n_moving, n_static, seed=seed, n_paths=n_paths, name="LandPolygons",
+                                    path_period=path_period, device_paths=device_paths)
+    ends = np.array([[w[0, 0], w[1, 0]] for w in scn.waypoints] + [[w[0, -1], w[1, -1]] for w in scn.waypoints])
+    scn.world_polygons = random_land(n_polygons, extent, seed=seed + 77, keep_clear=ends,
+                                     clear_margin=25.0 * np.sqrt(2.0) + LAND_CLEARANCE + 1.0)
     return scn
 
 

@@ -22,7 +22,7 @@ import torch
 
 from . import _lib
 from .config import Config
-from .scenarios import ScenarioSet
+from .scenarios import LAND_CLEARANCE, ScenarioSet
 from .spaces import Box, Dict as DictSpace
 
 
@@ -434,6 +434,7 @@ class AUVVecEnv:
             init_pos_jitter=50.0, mov_disp_std=500.0, mov_width_mean=10.0, mov_speed_lo=1.0, mov_speed_hi=3.0,
             st_disp_std=250.0, st_radius_mean=30.0,
             path_group=int(self.scenarios.path_group), path_period=int(self.scenarios.path_period or self.scenarios.n_scenarios),
+            land_clearance=LAND_CLEARANCE,
         )
 
     def regenerate_scenarios(self, ids: Optional[torch.Tensor] = None, seed: int = 0, epoch: int = 1):
@@ -441,10 +442,15 @@ class AUVVecEnv:
         movingobstacles.py:28-95 + helpers.py:5-35 with Philox streams keyed by (seed; scenario,
         slot, epoch)) into the listed pool slots (default: all) and refill their cached first
         observation.  Slots that a live env is running must not be listed -- see
-        ``refresh_finished``.  The host copy ``self.scenarios`` goes stale: ``pull_scenarios()``."""
+        ``refresh_finished``.  The host copy ``self.scenarios`` goes stale: ``pull_scenarios()``.
+
+        In a pool with a shared world of land polygons every placed object is also clear of land
+        (outside every polygon and farther than d from every ring): the vessel start by
+        ``scenarios.LAND_CLEARANCE``, a static circle's centre by its radius, a moving obstacle's track
+        start by its width; rejected draws are redrawn from the same stream.  Paths, goals and the later
+        course of moving obstacles are not tested.  A start area that stays covered after 4096 draws raises
+        in ``check_status()``."""
         M, Km = self.scenarios.n_scenarios, self.k_moving
-        if self.n_world:
-            raise NotImplementedError("scenario generation with a shared land-polygon world")
         if Km and self._pool["vel_table"].shape[0] < M * Km:
             raise ValueError("pool.vel_table must hold n_scenarios * k_moving entries (constant-velocity tracks)")
         gp = self.gen_params(seed, epoch)
@@ -595,6 +601,9 @@ class AUVVecEnv:
         st = int(self._scratch["status"].item())
         if st & _lib.STATUS_GEN_GAVE_UP:
             raise RuntimeError("scenario generator: an obstacle slot was still rejected after 100000 draws")
+        if st & _lib.STATUS_GEN_LAND_BLOCKED:
+            raise RuntimeError("scenario generator: a scenario's start area is covered by land "
+                               "(no vessel start clear of land after 4096 draws)")
         if st & _lib.STATUS_BOUNDS:
             raise RuntimeError("AUV_DEBUG_BOUNDS build: an index check inside a step kernel failed "
                                f"(source lines OR-ed together: {st >> 8})")

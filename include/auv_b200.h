@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define AUV_ABI_VERSION 20
+#define AUV_ABI_VERSION 21
 
 #define AUV_EINVAL (-1)  /* bad argument / NULL pointer / unsupported size */
 #define AUV_ENOTSUP (-2) /* feature not built */
@@ -76,6 +76,7 @@ extern "C" {
 #define AUV_STATUS_PATH_TOO_LONG 8 /* auv_pathbank_build: a path's 0.1 m polyline does not fit its slot (vcap) */
 #define AUV_STATUS_BOUNDS 16 /* -DAUV_DEBUG_BOUNDS builds only: an index check of a step kernel failed */
 #define AUV_STATUS_POLY_TOO_LARGE 4 /* a world polygon has more than AUV_MAX_POLY_VERTS vertices: it was skipped */
+#define AUV_STATUS_GEN_LAND_BLOCKED 32 /* scenario generator: no vessel start clear of land in 4096 draws (last one kept) */
 #ifndef AUV_PATH_STAGE_BLOCKS
 #define AUV_PATH_STAGE_BLOCKS 512
 #endif                            /* paths with at most this many projection blocks (~1.6 km) are searched from a
@@ -435,7 +436,14 @@ int auv_timer_read(AuvTimer* t, int slot, float* ms);
  * and of the goal), radius / width max(1, Poisson(mean)), and for moving obstacles direction
  * U(0, 2 pi) and speed U(lo, hi) -- for the listed scenarios of the pool, with counter-based
  * Philox4x32-10 streams keyed by (seed; scenario, slot, epoch): same arguments, same scenarios.
- * Every slot of a listed scenario is (re)generated as "used". */
+ * Every slot of a listed scenario is (re)generated as "used".
+ * In a pool with a shared world of land polygons (n_world > 0) every placed object must also be CLEAR OF
+ * LAND BY d -- outside every polygon (even-odd rule on the closed ring) and at an FP64 distance > d from
+ * every ring: the vessel start by gp->land_clearance (else jitter and heading are redrawn from the same
+ * stream; after 4096 draws AUV_STATUS_GEN_LAND_BLOCKED is raised and the last draw kept), a static circle's
+ * centre by its radius and a moving obstacle's track start by its width (both redrawn inside the rejection
+ * loop above).  Paths, goals and the later course of moving obstacles are not tested.  When no draw is
+ * rejected by land the Philox draws are those of a pool without a world. */
 typedef struct AuvGenParams {
   uint64_t seed;
   uint32_t epoch;               /* bump to draw a fresh scenario for the same pool slot      */
@@ -455,13 +463,17 @@ typedef struct AuvGenParams {
    * kernels then find whole CTAs on one path) */
   int32_t path_group;
   int32_t path_period;
+  /* pools with a shared land-polygon world (n_world > 0): the vessel start must be clear of land by
+   * land_clearance (0 = only outside every polygon).  See auv_generate_moving_obstacles. */
+  double land_clearance;
 } AuvGenParams;
 /* Writes path_id, vessel_init, mov_start, mov_width, mov_track, vel_table (entry m*Km+j), the
  * post-reset obstacle state mov_pos0/disp0/counter0, st_pos and st_radius of the scenarios
  * ids[0..n_ids) (device array; NULL = scenarios 0..n_ids-1).  The pool's arrays must be writable
  * device memory with vel_table holding n_scenarios * k_moving entries.  The reset cache of those
  * scenarios is stale afterwards: refill it with auv_reset + auv_observe(AUV_OBSERVE_RESET).
- * status (device int or NULL) receives AUV_STATUS_GEN_GAVE_UP. */
+ * status (device int or NULL) receives AUV_STATUS_GEN_GAVE_UP and AUV_STATUS_GEN_LAND_BLOCKED.  With
+ * n_world > 0 the pool's world_circle / world_voff / world_verts (and, when set, its grid) are read. */
 int auv_generate_moving_obstacles(const AuvGenParams* gp, const AuvPathBank* paths, const AuvScenarioPool* pool,
                                   const int32_t* ids, int n_ids, int32_t* status, void* stream);
 /* Fill the reset cache (pool.reset_obs / reset_max_progress / reset_mask) of n <= worker->n_envs
@@ -477,7 +489,9 @@ int auv_reset_cache_fill(const AuvConfig* cfg, const AuvRayTable* rays, const Au
  * `stream`: every env whose episode counter moved since the last call lists the slot it vacated
  * (at most `capacity` per call, the rest next time), those slots get freshly generated scenarios
  * (auv_generate_moving_obstacles semantics, Philox streams keyed by gp->seed / gp->epoch -- bump the
- * epoch per call) and their cached first observation is recomputed on the worker batch. */
+ * epoch per call) and their cached first observation is recomputed on the worker batch.  Pools with a
+ * shared land-polygon world are refreshed under the same land rule; live->status receives the generator's
+ * status bits. */
 typedef struct AuvRefreshScratch {
   int32_t* seen_episode; /* [N] episode counter of each env at the last call (zero-initialised)   */
   int32_t* ids;          /* [capacity] pool slots being regenerated (zero-initialised)            */
