@@ -8,7 +8,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("AUV_B200_LIB", os.path.join(_HERE, "libauv_b200.so"))  # override: tuning builds only
-ABI_VERSION = 21
+ABI_VERSION = 22
 REC_BYTES = 80
 MAX_POLY_VERTS = 192
 STATUS_REC_OVERFLOW = 1
@@ -193,7 +193,21 @@ class AuvStepOut(C.Structure):
         ("stats", _vp),
         ("seg_tests", _vp),
         ("episode_out", _vp),
+        ("tracks", _vp),  # const AuvTracks* (host pointer), NULL = no recording
     ]
+
+
+class AuvTracks(C.Structure):
+    _fields_ = [("count", C.c_int32), ("stride", C.c_int32), ("capacity", C.c_int32), ("reserved0", C.c_int32),
+                ("points", _vp), ("head", _vp), ("snap", _vp)]
+
+
+TRACK_HEAD_W = 8  # int32 per row head: episode, steps recorded, finished, collision, reached goal, scenario, obstacle updates, 0
+
+
+def track_snap_width(k_moving: int, k_static: int) -> int:
+    """doubles per snapshot row of AuvTracks.snap: path id, vessel_init, mov_lin records, st_rec records"""
+    return 4 + 8 * int(k_moving) + 4 * int(k_static)
 
 
 class AuvGenParams(C.Structure):
@@ -357,7 +371,7 @@ def load():
         raise AuvLibraryError(f"ABI mismatch: library {ver}, binding {ABI_VERSION}; rebuild")
     lib.auv_sizeof.argtypes = [C.c_int]
     for i, st in enumerate([AuvConfig, AuvRayTable, AuvPathBank, AuvScenarioPool, AuvBatch, AuvStepOut, AuvGenParams,
-                            AuvPathHdr, AuvRefreshScratch, AuvCompact, AuvPathBuild, AuvDelta]):
+                            AuvPathHdr, AuvRefreshScratch, AuvCompact, AuvPathBuild, AuvDelta, AuvTracks]):
         if lib.auv_sizeof(i) != C.sizeof(st):
             raise AuvLibraryError(f"struct layout mismatch for {st.__name__}: C {lib.auv_sizeof(i)} vs ctypes {C.sizeof(st)}")
     _lib = lib

@@ -51,14 +51,19 @@ class B200VecEnv:
     path_period=n)`` with ``fresh_scenarios=True`` draws a new MovingObstacles scenario for every episode on
     the GPU, as the reference's ``_generate()`` does at every ``reset()``.  ``record_history`` keeps the
     per-episode entries of ``env.history`` (environment.py:476-489) for ``get_attr("history")`` / the report.
+    ``record_tracks`` envs (spread evenly, ``impl.tracked_envs``) record their episodes on the GPU, up to
+    ``track_capacity`` steps each: ``get_attr("last_episode")`` returns the ``save_latest_episode`` dict of each
+    one's most recent finished episode (None for the other envs, and before a tracked env finished one).
     """
 
     def __init__(self, scenarios: ScenarioSet, num_envs: int, config: Optional[Config] = None, device="cuda:0",
                  test_mode: bool = False, fresh_scenarios: bool = False, refresh_every: int = 8, seed: int = 0,
-                 record_history: bool = True, history_limit: int = 100000, **vec_kw):
+                 record_history: bool = True, history_limit: int = 100000, record_tracks: int = 0,
+                 track_capacity: int = 2048, **vec_kw):
         from .vec_env import AUVVecEnv
 
-        self.impl = AUVVecEnv(scenarios, num_envs, config, device=device, test_mode=test_mode, auto_reset=True, **vec_kw)
+        self.impl = AUVVecEnv(scenarios, num_envs, config, device=device, test_mode=test_mode, auto_reset=True,
+                              record_tracks=record_tracks, track_capacity=track_capacity, **vec_kw)
         self.num_envs = int(num_envs)
         self.observation_space = self.impl.observation_space
         self.action_space = self.impl.action_space
@@ -125,6 +130,8 @@ class B200VecEnv:
             return [self._steps for _ in idx]
         if attr_name == "config":
             return [self.config for _ in idx]
+        if attr_name == "last_episode":  # reporting.plot_trajectory / plot_scenario input, per env
+            return [self.impl.last_episode(i) for i in idx]
         vals = self.impl.get_attr(attr_name).cpu().numpy()
         return [vals[i] for i in idx]
 

@@ -18,7 +18,8 @@
 //                      row by shared-memory atomicMin); WARP PER ENV for closeness / collision /
 //                      penalty / observation row / sector pooling / velocity channel; THREAD PER
 //                      ENV for reward, done, counters; a warp per finished env for the VecEnv
-//                      auto-reset (a COPY of the scenario's cached first observation)  FP32 issue
+//                      auto-reset (a COPY of the scenario's cached first observation); TRACK
+//                      twins also record the episode tracks of AuvStepOut.tracks    FP32 issue
 //   k_obstacle_update / k_vessel_step / k_reset   staged entry points
 //   k_pool_pack, k_obstacle_state                  pool packing / obstacle state read-back
 //   k_fma_probe        FP32 FMA peak micro-benchmark (roofline denominator)
@@ -779,6 +780,7 @@ struct LidarArgs {
   AuvScenarioPool pool;
   AuvBatch batch;
   AuvStepOut out;
+  const void* pad0;  // keeps the fields below 16-byte aligned, as before AuvStepOut.tracks (vector parameter loads)
   int mode;       // AUV_OBSERVE_STEP | AUV_OBSERVE_RESET
   int obs_dim;
   int e0, e1;     // envs [e0, e1) of the batch are processed by this launch
@@ -789,6 +791,7 @@ struct LidarArgs {
   double clear_closeness;  // -range * exp(-0.1 range): closeness reward when every ray is clear
   double inv_weight_sum;   // 1 / sum of the ray weights
   double feas_width;       // vessel_width * feasibility_width_multiplier (sensor.py:166-168)
+  AuvTracks trk;           // copy of *out.tracks (TRACK instantiations only; zeros otherwise)
 };
 
 // dynamic shared memory of a CTA; every part is 16-byte aligned
@@ -801,7 +804,8 @@ struct LidarSmem {
   float2* unit;     // [64]      cos/sin(2 pi k / 64) in FP32
   int* off;         // [E + 1]   exclusive scan of the envs' record counts
   float* pen;       // [E]       sum of w_i (penalty_i - clear penalty) over hit rays
-  int* flag;        // [E]       bit 0 collision, bit 1 auto-reset pending
+  int* flag;        // [E]       bit 0 collision, bit 1 auto-reset pending, (TRACK) bit 2 tracked env
+                    //           finished, bit 3 parity of its episode
   int* next;        // [E]       scenario the env resets onto
 };
 __host__ __device__ constexpr size_t lidar_smem_bytes_for(int E, int rpad, int vmax, int vel) {
@@ -952,7 +956,8 @@ __device__ __noinline__ void cast_long_polygon(const double2* __restrict__ wv, i
   }
 }
 
-template <bool COUNT, bool VEL, bool WORLD>
+// TRACK: record the episode tracks of AuvStepOut.tracks (instantiated with COUNT = false only)
+template <bool COUNT, bool VEL, bool WORLD, bool TRACK = false>
 __global__ void __launch_bounds__(AUV_LIDAR_THREADS, AUV_LIDAR_MINB) k_lidar(const __grid_constant__ LidarArgs A) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr int NW = AUV_LIDAR_THREADS / 32;
@@ -1311,6 +1316,18 @@ __global__ void __launch_bounds__(AUV_LIDAR_THREADS, AUV_LIDAR_MINB) k_lidar(con
         eo[1] = make_float4(reached ? 1.f : 0.f, (float)(cte_sum / (double)(t_step + 1)),
                             (float)A.paths.hdr[batch.env_pid[e]].length, (float)batch.episode[e]);
       }
+      if (TRACK && e % A.trk.stride == 0 && e / A.trk.stride < A.trk.count) {
+        // episode track: the point of this step and the row's head (row = parity of the episode,
+        // read before the auto-reset below moves the counter on)
+        const int ep = batch.episode[e];
+        const long long row = 2ll * (e / A.trk.stride) + (ep & 1);
+        reinterpret_cast<float4*>(A.trk.points)[row * A.trk.capacity + t_step % A.trk.capacity] =
+            make_float4((float)HAND(el, NAV_X), (float)HAND(el, NAV_Y), (float)HAND(el, NAV_PSI), (float)reward);
+        int4* hd = reinterpret_cast<int4*>(A.trk.head + 8 * row);
+        hd[0] = make_int4(ep, t_step + 1, done ? 1 : 0, collision ? 1 : 0);
+        hd[1] = make_int4(reached ? 1 : 0, scn, batch.obst_steps[e], 0);
+        if (done) fl = 4 | ((ep & 1) << 3);  // snapshot of the finished scenario in the bulk part
+      }
       if (!do_reset) {
         batch.cum_reward[e] = cum;
         batch.t_step[e] = t_step + 1;
@@ -1351,7 +1368,7 @@ __global__ void __launch_bounds__(AUV_LIDAR_THREADS, AUV_LIDAR_MINB) k_lidar(con
         batch.cte_sum[e] = 0.0;
         batch.max_progress[e] = A.pool.reset_max_progress[next];
         sm.next[el] = next;
-        fl = 2;
+        fl |= 2;
       }
     }
     sm.flag[el] = fl;
@@ -1359,8 +1376,28 @@ __global__ void __launch_bounds__(AUV_LIDAR_THREADS, AUV_LIDAR_MINB) k_lidar(con
   __syncthreads();
   // ---- auto-reset, bulk part (a warp per finished env): terminal obs out, cached first obs in,
   //      obstacle state (table-driven tracks only) and nearby list of the next scenario
+  //      (TRACK) and the snapshot of the scenario a tracked env finished: its pool slot still holds it
   for (int el = warp; el < ne; el += NW) {
-    if (!(sm.flag[el] & 2)) continue;
+    if (TRACK) {
+      const int tf = sm.flag[el];
+      if (!(tf & 6)) continue;
+      if (tf & 4) {
+        const int e = env0 + el, scn = (int)HAND(el, NAV_SCN);
+        const int km = A.pool.k_moving, ks = A.pool.k_static, w = 4 + 8 * km + 4 * ks;
+        double* sn = A.trk.snap + (2ll * (e / A.trk.stride) + ((tf >> 3) & 1)) * w;
+        for (int k = lane; k < w; k += 32) {
+          double v;
+          if (k == 0) v = (double)A.pool.path_id[scn];
+          else if (k < 4) v = A.pool.vessel_init[3ll * scn + (k - 1)];
+          else if (k < 4 + 8 * km) v = A.pool.mov_lin ? A.pool.mov_lin[8ll * km * scn + (k - 4)] : 0.0;
+          else v = A.pool.st_rec[4ll * ks * scn + (k - 4 - 8 * km)];
+          sn[k] = v;
+        }
+      }
+      if (!(tf & 2)) continue;
+    } else if (!(sm.flag[el] & 2)) {
+      continue;
+    }
     const int e = env0 + el, next = sm.next[el];
     const int km = A.pool.k_moving;
     float* obs = A.out.obs + (long long)e * A.obs_dim;
@@ -1591,6 +1628,7 @@ int auv_sizeof(int which) {
     case 9: return (int)sizeof(AuvCompact);
     case 10: return (int)sizeof(AuvPathBuild);
     case 11: return (int)sizeof(AuvDelta);
+    case 12: return (int)sizeof(AuvTracks);
     default: return AUV_EINVAL;
   }
 }
@@ -1693,10 +1731,27 @@ static int check_batch(const AuvConfig* cfg, const AuvScenarioPool* pool, const 
   return 0;
 }
 
+// AuvStepOut.tracks (NULL = no recording): checked before any device work
+static int check_tracks(const AuvStepOut* out, const AuvBatch* batch) {
+  const AuvTracks* t = out->tracks;
+  if (t == nullptr) return 0;
+  if (!t->points || !t->head || !t->snap) return set_err(AUV_EINVAL, "tracks: points / head / snap is NULL");
+  if (t->count < 1 || t->stride < 1 || t->capacity < 1)
+    return set_err(AUV_EINVAL, "tracks: count, stride and capacity must be >= 1");
+  if ((long long)(t->count - 1) * t->stride >= (long long)batch->n_envs)
+    return set_err(AUV_EINVAL, "tracks: (count - 1) * stride must be < n_envs");
+  if ((size_t)t->points & 15u) return set_err(AUV_EINVAL, "tracks: points must be 16-byte aligned");
+  if ((size_t)t->head & 15u) return set_err(AUV_EINVAL, "tracks: head must be 16-byte aligned");
+  if ((size_t)t->snap & 7u) return set_err(AUV_EINVAL, "tracks: snap must be 8-byte aligned");
+  if (out->seg_tests != nullptr) return set_err(AUV_EINVAL, "tracks cannot be recorded together with out.seg_tests");
+  return 0;
+}
+
 static int check_observe_args(const AuvConfig* cfg, const AuvRayTable* rays, const AuvPathBank* paths,
                               const AuvScenarioPool* pool, AuvBatch* batch, AuvStepOut* out, int mode) {
   if (int rc = check_cfg(cfg)) return rc;
   if (!paths || !pool || !batch || !out) return set_err(AUV_EINVAL, "NULL argument");
+  if (int rc = check_tracks(out, batch)) return rc;
   if (cfg->use_lidar && (!rays || !rays->unit64 || !rays->cos_sin || !rays->weight || !rays->sector))
     return set_err(AUV_EINVAL, "ray table is NULL with use_lidar");
   if (!out->obs) return set_err(AUV_EINVAL, "out.obs is NULL");
@@ -1765,11 +1820,13 @@ static int lidar_configure(size_t smem) {
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
   if (smem <= g_lidar_smem_configured[dev].load(std::memory_order_acquire)) return 0;
-  const void* fns[8] = {(const void*)auv::k_lidar<false, false, false>, (const void*)auv::k_lidar<true, false, false>,
-                        (const void*)auv::k_lidar<false, true, false>,  (const void*)auv::k_lidar<true, true, false>,
-                        (const void*)auv::k_lidar<false, false, true>,  (const void*)auv::k_lidar<true, false, true>,
-                        (const void*)auv::k_lidar<false, true, true>,   (const void*)auv::k_lidar<true, true, true>};
-  for (int i = 0; i < 8; ++i)
+  const void* fns[12] = {(const void*)auv::k_lidar<false, false, false>, (const void*)auv::k_lidar<true, false, false>,
+                         (const void*)auv::k_lidar<false, true, false>,  (const void*)auv::k_lidar<true, true, false>,
+                         (const void*)auv::k_lidar<false, false, true>,  (const void*)auv::k_lidar<true, false, true>,
+                         (const void*)auv::k_lidar<false, true, true>,   (const void*)auv::k_lidar<true, true, true>,
+                         (const void*)auv::k_lidar<false, false, false, true>, (const void*)auv::k_lidar<false, true, false, true>,
+                         (const void*)auv::k_lidar<false, false, true, true>,  (const void*)auv::k_lidar<false, true, true, true>};
+  for (int i = 0; i < 12; ++i)
     if (int rc = cuda_check(cudaFuncSetAttribute(fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
                             "cudaFuncSetAttribute(k_lidar)"))
       return rc;
@@ -1814,6 +1871,8 @@ static int launch_lidar(const AuvConfig* cfg, const AuvRayTable* rays, const Auv
   args.inv_log_range = (float)(1.0 / log1p(cfg->sensor_range));
   args.inv_weight_sum = (rays && rays->weight_sum > 0.0) ? 1.0 / rays->weight_sum : 0.0;
   args.feas_width = cfg->vessel_width * cfg->feasibility_width_multiplier;
+  const bool track = out->tracks != nullptr;  // validated by check_tracks: never together with seg_tests
+  if (track) args.trk = *out->tracks; else memset(&args.trk, 0, sizeof(args.trk));
   const size_t smem = lidar_smem_bytes(cfg, pool);
   if (int rc = lidar_configure(smem)) return rc;
   const int blocks = (cnt + args.envs_per_cta - 1) / args.envs_per_cta;
@@ -1821,7 +1880,13 @@ static int launch_lidar(const AuvConfig* cfg, const AuvRayTable* rays, const Auv
   const bool count = out->seg_tests != nullptr, vel = lidar_velocity(cfg) != 0;
   const bool world = pool->n_world > 0;  // the instantiation with the land-polygon path only when there is land
 #define AUV_LAUNCH_LIDAR(C, V, W) auv::k_lidar<C, V, W><<<blocks, AUV_LIDAR_THREADS, smem, s>>>(args)
-  if (world) {
+#define AUV_LAUNCH_LIDAR_TRACK(V, W) auv::k_lidar<false, V, W, true><<<blocks, AUV_LIDAR_THREADS, smem, s>>>(args)
+  if (track) {
+    if (world && vel) AUV_LAUNCH_LIDAR_TRACK(true, true);
+    else if (world) AUV_LAUNCH_LIDAR_TRACK(false, true);
+    else if (vel) AUV_LAUNCH_LIDAR_TRACK(true, false);
+    else AUV_LAUNCH_LIDAR_TRACK(false, false);
+  } else if (world) {
     if (count && vel) AUV_LAUNCH_LIDAR(true, true, true);
     else if (count) AUV_LAUNCH_LIDAR(true, false, true);
     else if (vel) AUV_LAUNCH_LIDAR(false, true, true);
@@ -1833,6 +1898,7 @@ static int launch_lidar(const AuvConfig* cfg, const AuvRayTable* rays, const Auv
     else AUV_LAUNCH_LIDAR(false, false, false);
   }
 #undef AUV_LAUNCH_LIDAR
+#undef AUV_LAUNCH_LIDAR_TRACK
   return cuda_check(cudaGetLastError(), "k_lidar");
 }
 
@@ -2069,6 +2135,7 @@ static int step_host_chunked(const AuvConfig* cfg, const AuvRayTable* rays, cons
     key = fnv1a(key, pool, sizeof(*pool));
     key = fnv1a(key, batch, sizeof(*batch));
     key = fnv1a(key, out, sizeof(*out));
+    if (out->tracks) key = fnv1a(key, out->tracks, sizeof(*out->tracks));
     const void* ptrs[6] = {actions_host, actions_dev, obs_host, reward_host, done_host, (const void*)(size_t)n_chunks};
     key = fnv1a(key, ptrs, sizeof(ptrs));
     if (cb) key = fnv1a(key, cb, sizeof(*cb));
@@ -2258,6 +2325,7 @@ int auv_step_host(const AuvConfig* cfg, const AuvRayTable* rays, const AuvPathBa
                   uint8_t* done_host, void* stream) {
   if (!cfg || !batch || !out || !actions_host || !actions_dev || !obs_host || !reward_host || !done_host)
     return set_err(AUV_EINVAL, "NULL argument");
+  if (int rc = check_tracks(out, batch)) return rc;  // before the copy of the actions
   cudaStream_t s = (cudaStream_t)stream;
   const size_t n = (size_t)batch->n_envs;
   if (int rc = cuda_check(cudaMemcpyAsync(actions_dev, actions_host, n * 2 * sizeof(float),

@@ -131,7 +131,8 @@ class AUVEnv:
         if self._vec is None or (self._block_pos >= self.scenario.n_scenarios and not self._recycle):
             self.scenario, self._recycle = self._generate_block(self.block_size)
             self._vec = AUVVecEnv(self.scenario, 1, self.config, device=self.device, test_mode=self.test_mode,
-                                  auto_reset=False, debug=True)
+                                  auto_reset=False, debug=True, count_ray_tests=False, record_tracks=1,
+                                  track_capacity=max(1, int(self.config.episode.max_timesteps)))
             self.vec_env_builds += 1
             self.rewarder = SimpleNamespace(params=dict(REWARDER_PARAMS[self.scenario.rewarder]))
             self._block_pos, self._idx = 1, 0
@@ -223,9 +224,18 @@ class AUVEnv:
         return self.scenario.describe(self._idx)
 
     def save_latest_episode(self, save_history=True):
-        """environment.py:466-489 (path_taken histories are not kept: SURVEY B11)."""
-        self.last_episode = {"path": self.path(np.linspace(0, self.path.length, 1000)), "path_taken": None,
-                             "obstacles": self.obstacles}
+        """environment.py:466-489.  ``path_taken`` and the obstacles' histories are the episode track the step
+        kernel recorded (``AUVVecEnv.current_episode``: reset() saves whatever episode was running).  The track
+        holds ``max_timesteps`` steps; a longer episode (``test_mode`` has no time limit) keeps its last
+        ``max_timesteps`` rows: ``truncated`` is then True and ``step_index`` numbers the rows (row 0 is not
+        the initial pose)."""
+        rec = self._vec.current_episode(0)
+        obstacles = dict(self.obstacles, moving_path_taken=rec["obstacles"]["moving_path_taken"])
+        self.last_episode = {"path": self.path(np.linspace(0, self.path.length, 1000)), "path_taken": rec["path_taken"],
+                             "heading_taken": rec["heading_taken"], "rewards": rec["rewards"], "obstacles": obstacles,
+                             "truncated": rec["truncated"]}
+        if rec["truncated"]:
+            self.last_episode["step_index"] = rec["step_index"]
         if save_history:
             t = self.t_step
             self.history.append({

@@ -151,6 +151,72 @@ def advance_obstacles(scn: ScenarioSet, pos, counter, dt):
     return np.where(used, pos + disp, pos), np.where(used, disp, 0.0), np.where(used[..., 0], counter, 0.0)
 
 
+def _two_sum(a, b):
+    """s + e == a + b exactly, s = RN(a + b) (Knuth)."""
+    s = a + b
+    bb = s - a
+    return s, (a - (s - bb)) + (b - bb)
+
+
+def _fma(a, b, c):
+    """Correctly rounded a * b + c element-wise -- the device's fma -- vectorised: a * b is split exactly into
+    uh + ul (Dekker's product), c + uh into th + tl (TwoSum), tl + ul is rounded to odd, and th plus that is
+    rounded to nearest once (Boldo & Melquiond, "Emulation of FMA and correctly rounded sums: proved
+    algorithms using rounding to odd", IEEE TC 57(4), 2008; exact barring overflow / underflow)."""
+    a, b, c = np.broadcast_arrays(np.asarray(a, np.float64), np.asarray(b, np.float64), np.asarray(c, np.float64))
+    split = 134217729.0  # 2^27 + 1
+    t = split * a
+    ah = t - (t - a)
+    al = a - ah
+    t = split * b
+    bh = t - (t - b)
+    bl = b - bh
+    uh = a * b
+    ul = ((ah * bh - uh) + ah * bl + al * bh) + al * bl
+    th, tl = _two_sum(c, uh)
+    v, ve = _two_sum(tl, ul)
+    # round to odd: an inexact v with an even significand moves one ulp towards the exact sum
+    fix = (ve != 0) & ((v.view(np.int64) & 1) == 0)
+    v = np.where(fix, np.nextafter(v, np.where(ve > 0, np.inf, -np.inf)), v)
+    return th + v
+
+
+def linear_track_positions(rec, n, first_wrap: int, wrap_period: int):
+    """Positions of constant-velocity obstacle tracks after ``n`` updates since reset -- the closed form
+    of obstacles.py:195-215 that the step and ``auv_obstacle_state`` evaluate (AuvScenarioPool.linear_tracks):
+        n <  first_wrap : pos0 + n d
+        n >= first_wrap : start + ((n - first_wrap) mod wrap_period + 1) d
+    ``rec`` [k, 8] packed pool.mov_lin records (pos0, d, width, start, 0), ``n`` int array [S].
+    Returns [S, k, 2], FP64 with fused multiply-adds: bit-identical to the device."""
+    rec = np.asarray(rec, np.float64).reshape(-1, 8)
+    n = np.asarray(n, np.int64).reshape(-1, 1, 1)
+    wrapped = n >= first_wrap
+    m = np.where(wrapped, (n - first_wrap) % wrap_period + 1, n).astype(np.float64)
+    base = np.where(wrapped, rec[None, :, 5:7], rec[None, :, 0:2])
+    return _fma(m, rec[None, :, 2:4], base)
+
+
+def table_track_positions(scn: ScenarioSet, m: int, n, dt: float):
+    """Positions of the moving obstacles of pool scenario ``m`` after ``n`` updates since reset ([S] ints,
+    non-decreasing not required): ``initial_obstacle_state`` followed by ``advance_obstacles`` step by step.
+    Returns [S, Km, 2]."""
+    from types import SimpleNamespace
+
+    one = SimpleNamespace(mov_start=scn.mov_start[m], mov_width=scn.mov_width[m], mov_track=scn.mov_track[m],
+                          vel_table=scn.vel_table, post_generate_update=scn.post_generate_update)
+    pos, _, counter = ScenarioSet.initial_obstacle_state(one, dt)
+    n = np.asarray(n, np.int64).reshape(-1)
+    out = np.zeros((n.size, one.mov_width.shape[0], 2))
+    order = np.argsort(n, kind="stable")
+    u = 0
+    for k in order:
+        while u < n[k]:
+            pos, _, counter = advance_obstacles(one, pos, counter, dt)
+            u += 1
+        out[k] = pos
+    return out
+
+
 def _empty_moving(M):
     return (
         np.zeros((M, 0, 2)),

@@ -22,7 +22,7 @@ import torch
 
 from . import _lib
 from .config import Config
-from .scenarios import LAND_CLEARANCE, ScenarioSet
+from .scenarios import LAND_CLEARANCE, ScenarioSet, linear_track_positions, table_track_positions
 from .spaces import Box, Dict as DictSpace
 
 
@@ -83,6 +83,86 @@ def make_auv_config(cfg: Config, rewarder: str, test_mode: bool, auto_reset: boo
     )
 
 
+def pick_finished_row(head) -> Optional[int]:
+    """Row (0 / 1) of a track slot's ``head`` [2, 8] that holds the most recent finished episode: of the
+    rows whose finished flag is set, the one with the greater episode number; None if neither is."""
+    head = np.asarray(head)
+    rows = [p for p in (0, 1) if head[p, 2]]
+    if not rows:
+        return None
+    return max(rows, key=lambda p: int(head[p, 0]))
+
+
+def track_rows(head_row, points_row, capacity: int):
+    """The recorded points of one track row in step order: (points [n, 4], step_index [n] = steps taken
+    after each point, truncated).  An episode longer than ``capacity`` keeps its last ``capacity`` points."""
+    n, T = int(head_row[1]), int(capacity)
+    pts = np.asarray(points_row)
+    if n <= T:
+        return pts[:n].copy(), np.arange(1, n + 1), False
+    t = np.arange(n - T, n)
+    return pts[t % T].copy(), t + 1, True
+
+
+def assemble_episode(head_row, points_row, snap_row, capacity: int, k_moving: int, k_static: int, dt: float,
+                     linear: Optional[dict], scenarios: Optional[ScenarioSet], path_table=None, polygons=()):
+    """The ``save_latest_episode`` dict (environment.py:466-489) of one track row: ``head_row`` [8],
+    ``points_row`` [T, 4] and the scenario snapshot ``snap_row`` [4 + 8 k_moving + 4 k_static] (layout of
+    AuvTracks in include/auv_b200.h).  ``linear``: the pool's closed-form track constants (``AUVVecEnv.linear``)
+    or None for table-driven pools, whose tracks are re-run from ``scenarios`` (slot = the row's scenario id).
+    ``path_table(path_id)`` evaluates the path (None: no ``"path"``)."""
+    snap = np.asarray(snap_row, np.float64)
+    pts, step_index, truncated = track_rows(head_row, points_row, capacity)
+    n = int(head_row[1])
+    init = snap[1:4].copy()
+    if truncated:
+        xy, psi, steps = pts[:, 0:2].astype(np.float64), pts[:, 2].astype(np.float64), step_index
+    else:
+        xy = np.concatenate([init[None, 0:2], pts[:, 0:2].astype(np.float64)], axis=0)
+        psi = np.concatenate([init[2:3], pts[:, 2].astype(np.float64)])
+        steps = np.arange(n + 1)
+    pid = int(snap[0])
+    km, ks = int(k_moving), int(k_static)
+    mov = None
+    updates = int(head_row[6]) - (n - steps)  # obstacle updates since reset at each row
+    moving_taken = np.zeros((len(steps), 0, 2))
+    if km:
+        rec = snap[4:4 + 8 * km].reshape(km, 8)
+        if linear is not None:
+            used = rec[:, 4] > 0
+            moving_taken = linear_track_positions(rec[used], updates, linear["first_wrap"], linear["wrap_period"])
+            d = rec[used, 2:4]
+            mov = dict(width=rec[used, 4].copy(), start=rec[used, 5:7].copy(),
+                       vel_tables=[np.repeat(v[None] / dt, linear["vel_len"], axis=0) for v in d])
+        else:
+            m = int(head_row[5])
+            used = scenarios.mov_width[m] > 0
+            moving_taken = table_track_positions(scenarios, m, updates, dt)[:, used]
+            mov = scenarios.describe(m)["moving"]
+    st = None
+    if ks:
+        sr = snap[4 + 8 * km:].reshape(ks, 4)
+        used = sr[:, 2] > 0
+        st = dict(pos=sr[used, 0:2].copy(), radius=sr[used, 2].copy())
+    obstacles = dict(
+        waypoints=scenarios.waypoints[pid] if scenarios is not None else None, vessel_init=init, moving=mov, static=st,
+        rewarder=scenarios.rewarder if scenarios is not None else None,
+        post_generate_update=scenarios.post_generate_update if scenarios is not None else None,
+        polygons=list(polygons), moving_path_taken=moving_taken,
+    )
+    ep = dict(
+        path=None, path_taken=xy, heading_taken=psi, rewards=pts[:, 3].astype(np.float64), obstacles=obstacles,
+        episode=int(head_row[0]), timesteps=n, collision=bool(head_row[3]), reached_goal=bool(head_row[4]),
+        truncated=bool(truncated), scenario=int(head_row[5]), path_id=pid,
+    )
+    if truncated:
+        ep["step_index"] = steps
+    if path_table is not None:
+        tab = path_table(pid)
+        ep["path"] = tab(np.linspace(0, tab.length, 1000))
+    return ep
+
+
 class AUVVecEnv:
     """N gym-auv environments stepped together on one GPU.
 
@@ -96,6 +176,7 @@ class AUVVecEnv:
     test_mode : as BaseEnvironment(test_mode=...) (environment.py:32,380-382)
     auto_reset: VecEnv semantics (default) or manual ``reset_envs``
     debug     : also record per-ray distances, culling windows and FP64 navigation values
+    count_ray_tests : count the reference-semantics ray/segment tests (get_attr("seg_tests")); default: ``debug``
     sector_outputs : also produce per-sector min-pooled and feasibility-pooled ranges
                      (get_attr("sector_min_dist") / get_attr("sector_feasible_dist"))
     chunks    : > 1 cuts the batch into that many env ranges which run their kernels on
@@ -122,6 +203,12 @@ class AUVVecEnv:
     linear_tracks : "auto" (default) = pools whose moving obstacles all follow constant-velocity tracks
                 (the MovingObstacles family) are stepped with the closed form of the update and keep no
                 per-env obstacle state; False forces the general table-driven update
+    record_tracks : record the episode tracks (path_taken, headings, rewards, the scenario) of this many envs,
+                spread evenly (stride N // record_tracks; indices in ``tracked_envs``), in the step kernel:
+                ``last_episode(i)`` / ``current_episode(i)``.  0 (default) = off.  The ray-test counting
+                kernels do not record: with ``debug`` pass ``count_ray_tests=False`` (else ValueError); the env
+                then has no ``seg_tests`` output
+    track_capacity : steps kept per recorded episode; a longer episode keeps its last ``track_capacity``
     """
 
     def __init__(
@@ -148,6 +235,9 @@ class AUVVecEnv:
         host_threads: Optional[int] = None,
         host_transfer: Optional[str] = None,
         delta_gran: int = 16,
+        record_tracks: int = 0,
+        track_capacity: int = 2048,
+        count_ray_tests: Optional[bool] = None,
         _shared: Optional[dict] = None,
     ):
         self.device = torch.device(device)
@@ -335,13 +425,36 @@ class AUVVecEnv:
         if debug:
             self._out["lidar_dist"] = z((N, max(R, 1)), torch.float32)
             self._out["windows"] = z((N, max(K, 1), 2), torch.int32)
+        count_ray_tests = bool(debug) if count_ray_tests is None else bool(count_ray_tests)
+        if count_ray_tests and int(record_tracks) > 0:
+            raise ValueError("record_tracks cannot be combined with the ray-test counter of debug: "
+                             "pass count_ray_tests=False")
+        if int(record_tracks) > 0:
+            del self._out["seg_tests"]  # not counted: get_attr("seg_tests") raises instead of reading 0
         o = self._out
         ptr = lambda k: o[k].data_ptr() if k in o else None
+        # episode tracks of a sample of the envs (AuvTracks), recorded by the step kernel
+        self.record_tracks = Kt = max(0, min(int(record_tracks), N))
+        self.track_capacity = T = int(track_capacity)
+        self.tracked_envs = np.zeros(0, dtype=np.int64)
+        self._tracks, self.tracks = None, None
+        if Kt:
+            if T < 1:
+                raise ValueError("track_capacity must be >= 1")
+            stride = N // Kt
+            self.tracked_envs = np.arange(Kt, dtype=np.int64) * stride
+            W = _lib.track_snap_width(Km, Ks)
+            self._tracks = dict(points=z((Kt, 2, T, 4), torch.float32), head=z((Kt, 2, _lib.TRACK_HEAD_W), torch.int32),
+                                snap=z((Kt, 2, W), torch.float64), stride=stride)
+            tk = self._tracks
+            self.tracks = _lib.AuvTracks(Kt, stride, T, 0, tk["points"].data_ptr(), tk["head"].data_ptr(),
+                                         tk["snap"].data_ptr())
         self.out = _lib.AuvStepOut(
             ptr("obs"), ptr("reward"), ptr("done"), ptr("collision"), ptr("reached_goal"), ptr("goal_distance"),
             ptr("progress"), ptr("lidar_dist"), ptr("windows"), ptr("terminal_obs"), ptr("sector_min_dist"),
             ptr("sector_feasible_dist"), ptr("stats"),
-            ptr("seg_tests") if debug else None, ptr("episode_out"),
+            ptr("seg_tests") if count_ray_tests else None, ptr("episode_out"),
+            C.addressof(self.tracks) if Kt else None,
         )
         self.actions_dev = z((N, 2), torch.float32)
         self._pinned = None
@@ -454,6 +567,7 @@ class AUVVecEnv:
         if Km and self._pool["vel_table"].shape[0] < M * Km:
             raise ValueError("pool.vel_table must hold n_scenarios * k_moving entries (constant-velocity tracks)")
         gp = self.gen_params(seed, epoch)
+        self._pool["host_stale"] = True  # the host ScenarioSet no longer describes every pool slot
         idp, n = None, M
         if ids is not None:
             ids = ids.to(self.device, torch.int32).contiguous()
@@ -473,7 +587,9 @@ class AUVVecEnv:
         auv_random_curve_waypoints + auv_pathbank_build) into the listed slots of a device-built bank
         (default: all).  Scenarios that follow those paths are stale afterwards -- regenerate them
         (``regenerate_scenarios``) before the next ``reset()``; ``MovingObstacles._generate`` does the same
-        pair of draws per episode (movingobstacles.py:28-95)."""
+        pair of draws per episode (movingobstacles.py:28-95).  The ``"path"`` of a recorded episode
+        (``last_episode``) is evaluated from the bank when it is read, so it is stale for an episode
+        whose path slot was replaced here."""
         from .pathbank import DevicePathBank
 
         bank = self.scenarios.bank
@@ -549,6 +665,7 @@ class AUVVecEnv:
         rs["epoch"] += 1
         self._gen_epoch = rs["epoch"]
         gp = self.gen_params(seed, rs["epoch"])
+        self._pool["host_stale"] = True
         cfg, rays, paths, pool, batch = self._refs()
         with torch.cuda.device(self.device):
             _lib.check(self.lib.auv_refresh_finished(cfg, rays, paths, pool, batch, C.byref(w.batch), C.byref(w.out),
@@ -781,6 +898,8 @@ class AUVVecEnv:
         kw.setdefault("host_chunks", max(1, self.host_chunks // int(n_groups)))
         kw.setdefault("host_transfer", self.host_transfer)
         kw.setdefault("delta_gran", self.delta_gran)
+        kw.setdefault("record_tracks", self.record_tracks)
+        kw.setdefault("track_capacity", self.track_capacity)
         return [AUVVecEnv(self.scenarios, n, self.config, device=self.device, test_mode=self.test_mode,
                           auto_reset=bool(self.cfg.auto_reset), cull_mode=self._cull_mode, env_offset=g * n,
                           max_nearby=self._max_nearby, velocity_mode=self._velocity_mode,
@@ -881,6 +1000,82 @@ class AUVVecEnv:
                 "auv_observe",
             )
         return self._out["obs"]
+
+    # ------------------------------------------------------------------ episode tracks (record_tracks)
+    def _track_slot(self, i: int) -> Optional[int]:
+        if self._tracks is None:
+            return None
+        i, stride = int(i), self._tracks["stride"]
+        if i < 0 or i % stride or i // stride >= self.record_tracks:
+            return None
+        return i // stride
+
+    def _track_sync(self):
+        torch.cuda.current_stream(self.device).synchronize()
+        if getattr(self, "_async_stream", None) is not None:
+            self._async_stream.synchronize()
+
+    def _path_table(self, pid: int):
+        from .pathbank import DevicePathBank, build_path
+
+        bank = self.scenarios.bank
+        if isinstance(bank, DevicePathBank) and bank._tables is None:  # one path, not the whole bank
+            return build_path(bank.waypoints[pid])
+        return bank.tables[pid]
+
+    def _assemble(self, head_row, points_row, snap_row):
+        if self.linear is None and self.k_moving and self._pool.get("host_stale"):
+            # table-driven histories are re-run from the host ScenarioSet (snapshots hold no velocity tables)
+            raise RuntimeError("obstacle histories of a table-driven pool are rebuilt from the host scenarios, which "
+                               "GPU scenario generation has made stale: record tracks with linear_tracks='auto' "
+                               "on generated pools")
+        return assemble_episode(head_row, points_row, snap_row, self.track_capacity, self.k_moving, self.k_static,
+                                float(self.config.simulation.t_step_size), self.linear, self.scenarios,
+                                self._path_table, self.scenarios.world_polygons)
+
+    def last_episode(self, i: int) -> Optional[dict]:
+        """The most recent FINISHED episode of env ``i`` as ``BaseEnvironment.save_latest_episode`` stores it
+        (environment.py:466-489): ``path``, ``path_taken`` [n + 1, 2] (row 0 = the scenario's vessel_init, the
+        other rows the recorded FP32 positions after each step), ``heading_taken`` [n + 1], ``rewards`` [n],
+        ``obstacles`` (``ScenarioSet.describe``-shaped, from the scenario snapshot taken when the episode
+        ended, plus ``moving_path_taken`` [n + 1, k_used, 2]), ``episode``, ``timesteps``, ``collision``,
+        ``reached_goal``, ``truncated`` (episode longer than ``track_capacity``: the last ``track_capacity``
+        rows are kept, numbered by ``step_index``).  None when env ``i`` is not tracked or has finished no
+        episode.  Synchronises the env's stream; copies one track slot."""
+        slot = self._track_slot(i)
+        if slot is None:
+            return None
+        self._track_sync()
+        tk = self._tracks
+        head = tk["head"][slot].cpu().numpy()
+        p = pick_finished_row(head)
+        if p is None:
+            return None
+        return self._assemble(head[p], tk["points"][slot, p].cpu().numpy(), tk["snap"][slot, p].cpu().numpy())
+
+    def current_episode(self, i: int) -> Optional[dict]:
+        """``last_episode``'s dict for the episode env ``i`` is running now (finished or not: without
+        auto-reset a finished env stays on its episode until reset), read from its live pool slot -- which a
+        refresh never regenerates while the env runs it.  None when env ``i`` is not tracked."""
+        slot = self._track_slot(i)
+        if slot is None:
+            return None
+        self._track_sync()
+        tk, i = self._tracks, int(i)
+        ep, scn = int(self._st["episode"][i].item()), int(self._st["scn_id"][i].item())
+        p = ep & 1
+        head = tk["head"][slot, p].cpu().numpy()
+        if int(head[0]) != ep or int(head[1]) == 0:  # no step of this episode yet: the row is stale
+            head = np.array([ep, 0, 0, 0, 0, scn, 0, 0], dtype=np.int32)
+        pool, km, ks = self._pool, self.k_moving, self.k_static
+        parts = [pool["path_id"][scn:scn + 1].to(torch.float64), pool["vessel_init"][scn]]
+        if km:
+            parts.append(pool["mov_lin"][scn].reshape(-1) if "mov_lin" in pool
+                         else torch.zeros(8 * km, dtype=torch.float64, device=self.device))
+        if ks:
+            parts.append(pool["st_rec"][scn, :ks].reshape(-1))
+        snap = torch.cat(parts).cpu().numpy()
+        return self._assemble(head, tk["points"][slot, p].cpu().numpy(), snap)
 
     # ------------------------------------------------------------------ attributes the reference driver reads
     @property

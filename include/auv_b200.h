@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define AUV_ABI_VERSION 21
+#define AUV_ABI_VERSION 22
 
 #define AUV_EINVAL (-1)  /* bad argument / NULL pointer / unsupported size */
 #define AUV_ENOTSUP (-2) /* feature not built */
@@ -265,6 +265,33 @@ typedef struct AuvBatch {
   int32_t* env_pid;       /* [N] pool.path_id[scn_id[e]], cached by reset                       */
 } AuvBatch;
 
+/* Episode tracks of a sample of the batch (the path_taken / obstacle histories of
+ * BaseEnvironment.save_latest_episode, environment.py:466-489), recorded by the step kernel.
+ * Env e is tracked iff e % stride == 0 && e / stride < count; its track slot is t = e / stride.
+ * Each slot has two rows, p = 0 and 1: an episode with counter ep (AuvBatch.episode before any
+ * reset in the step) writes row p = ep & 1, so the row of the episode an env just finished stays
+ * intact for the whole of its next episode, which writes the other row.  Every AUV_OBSERVE_STEP
+ * writes, for each tracked env, the point of the step and rewrites the row's head; the step in
+ * which the episode ends also copies the scenario it ran on into the row's snapshot (the pool slot
+ * may be regenerated later, auv_refresh_finished).  All buffers are device memory.
+ *   points [count][2][capacity] float4: x, y, psi after the step, reward of the step, at index
+ *          t_step % capacity (t_step = steps before this one): an episode longer than capacity
+ *          keeps its last capacity points
+ *   head   [count][2][8] int32: episode counter, steps recorded (t_step + 1), finished flag,
+ *          collision, reached goal, scenario id, obstacle updates since reset, 0
+ *   snap   [count][2][4 + 8 k_moving + 4 k_static] double: pool path_id, vessel_init (3), then each
+ *          moving slot's pool.mov_lin record (8; zeros without linear_tracks) and each static slot's
+ *          pool.st_rec record (4) -- valid once the row's finished flag is set */
+typedef struct AuvTracks {
+  int32_t count;    /* K >= 1 tracked envs                                             */
+  int32_t stride;   /* >= 1, (count - 1) * stride < n_envs                             */
+  int32_t capacity; /* T >= 1 points kept per episode                                  */
+  int32_t reserved0;
+  float* points;    /* 16-byte aligned (one float4 store per point)                   */
+  int32_t* head;    /* 16-byte aligned (a row is written as two 16-byte stores)        */
+  double* snap;     /* 8-byte aligned                                                  */
+} AuvTracks;
+
 /* Outputs of one step / observe (all optional except obs/reward/done). */
 typedef struct AuvStepOut {
   float* obs;            /* [N][obs_dim]  obs_dim = 6 (+ n_sensors (+ 2 n_sensors))     */
@@ -287,6 +314,12 @@ typedef struct AuvStepOut {
                             episode an env finished in this step (rows of envs with done = 1):
                             reward, timesteps, progress, collision, reached_goal, mean
                             cross-track error, path length, episode number                      */
+  const AuvTracks* tracks; /* HOST pointer to the track descriptor, or NULL = no recording: a
+                            zero-initialised AuvStepOut records nothing.  Validated by every step
+                            entry point before any device work (AUV_EINVAL): NULL buffers, count /
+                            stride / capacity < 1, (count - 1) * stride >= n_envs, misaligned
+                            points / head / snap, and tracks together with seg_tests (the ray-test
+                            counting kernels do not record: set one or the other)              */
 } AuvStepOut;
 
 /* indices into AuvStepOut.stats (mirrors env.history keys, environment.py:476-489) */
@@ -309,7 +342,7 @@ typedef struct AuvStepOut {
 int auv_abi_version(void);
 /* sizeof of the ABI structs, in declaration order (0 AuvConfig, 1 AuvRayTable, 2 AuvPathBank,
  * 3 AuvScenarioPool, 4 AuvBatch, 5 AuvStepOut, 6 AuvGenParams, 7 AuvPathHdr, 8 AuvRefreshScratch, 9 AuvCompact,
- * 10 AuvPathBuild, 11 AuvDelta) so a binding
+ * 10 AuvPathBuild, 11 AuvDelta, 12 AuvTracks) so a binding
  * can verify its layout. */
 int auv_sizeof(int which);
 const char* auv_last_error(void);
