@@ -7,7 +7,8 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("AUV_B200_LIB", os.path.join(_HERE, "libauv_b200.so"))  # override: tuning builds only
+# AUV_B200_LIB loads a library built elsewhere, e.g. the -DAUV_DEBUG_BOUNDS build of the tests
+LIB_PATH = os.environ.get("AUV_B200_LIB", os.path.join(_HERE, "libauv_b200.so"))
 ABI_VERSION = 22
 REC_BYTES = 80
 MAX_POLY_VERTS = 192
@@ -245,7 +246,7 @@ class AuvCompact(C.Structure):
 
 
 class AuvDelta(C.Structure):
-    _fields_ = [("obs_host", _vp), ("shadow", _vp), ("shipped", _vp), ("gran", C.c_int32), ("ctas", C.c_int32)]
+    _fields_ = [("obs_host", _vp), ("shadow", _vp), ("shipped", _vp), ("gran", C.c_int32), ("reserved0", C.c_int32)]
 
 
 EXPORTS = [

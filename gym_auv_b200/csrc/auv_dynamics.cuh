@@ -12,11 +12,9 @@ struct S6 {
   double x, y, psi, u, v, r;
 };
 
-// nu_dot = M^-1 (tau - D nu - N(nu) nu) and eta_dot = Rz(psi) nu with cos/sin(psi) supplied
-#ifndef AUV_RK_INLINE
-#define AUV_RK_INLINE __forceinline__  // (out of line was measured: 0.104 -> 0.126 ms, the S6 structs go through the stack)
-#endif
-__device__ AUV_RK_INLINE S6 state_dot_cs(const S6& s, double cp, double sp, double tau_u, double tau_r) {
+// nu_dot = M^-1 (tau - D nu - N(nu) nu) and eta_dot = Rz(psi) nu with cos/sin(psi) supplied.
+// Inlined, as rot_cs below: out of line was measured at 0.104 -> 0.126 ms (the S6 structs go through the stack)
+__device__ __forceinline__ S6 state_dot_cs(const S6& s, double cp, double sp, double tau_u, double tau_r) {
   // M = [[25.8,0,0],[0,33.8,1.0948],[0,1.0948,2.76]]   (constants.py:33-36)
   constexpr double m11 = 33.8, m12 = 23.8 * 0.046, m22 = 2.76;
   constexpr double det = m11 * m22 - m12 * m12;
@@ -40,7 +38,7 @@ __device__ AUV_RK_INLINE S6 state_dot_cs(const S6& s, double cp, double sp, doub
 // psi0 + h * (combination of yaw rates), a small offset from the step's initial heading, so one
 // FP64 sincos per step replaces six (+ six fmod in princip); results agree with
 // sincos(princip(psi0 + d)) to ~2e-16.  Larger offsets take the direct route.
-__device__ AUV_RK_INLINE void rot_cs(double c0, double s0, double psi0, double d, double& c, double& s) {
+__device__ __forceinline__ void rot_cs(double c0, double s0, double psi0, double d, double& c, double& s) {
   if (fabs(d) > 0.5) {
     sincos(princip(psi0 + d), &s, &c);
     return;

@@ -352,9 +352,6 @@ __device__ __forceinline__ bool slot_is_near(const AuvScenarioPool& pool, const 
   return (dist - width) < range;
 }
 
-#ifndef AUV_CULL_COOP
-#define AUV_CULL_COOP 1
-#endif
 // Culling stage for one env by its group of G lanes: the lanes take different obstacle slots
 // (slot j of a 32-slot word belongs to lane j % G), records are emitted in slot order by a
 // ballot prefix.  `store` is false for the padding groups past the end of the env range.
@@ -375,11 +372,10 @@ __device__ __forceinline__ void cull_env_group(const AuvConfig& cfg, const AuvSc
   // An env refreshes its list every 25 steps; in the desynchronised steady state that is ~1 of the 8 envs of a
   // warp per step -- but most warps have one.  The warp therefore does its refreshing envs one after the other
   // with ALL 32 lanes on different slots (one round for 32 slots) instead of leaving each to the 4 lanes of its
-  // group (8 rounds during which the other groups wait).  (AUV_CULL_COOP 0: the per-group version.)
+  // group (8 rounds during which the other groups wait).
   const int K = pool.k_moving + pool.k_static;
   const bool grid = pool.world_cell_off != nullptr && pool.n_world > 0;  // world slots through the broad phase
   const int S_scan = grid ? K : S;
-#if AUV_CULL_COOP
   const unsigned rmask = __ballot_sync(AUV_FULL, refresh && sub == 0 && store);
   for (unsigned rm = rmask; rm; rm &= rm - 1) {  // uniform in the warp
     const int src = __ffs(rm) - 1;
@@ -396,22 +392,7 @@ __device__ __forceinline__ void cull_env_group(const AuvConfig& cfg, const AuvSc
     }
   }
   if (rmask) __syncwarp();
-#endif
   if (refresh) {
-#if !AUV_CULL_COOP
-    for (int base = 0; base < S; base += 32) {
-      unsigned word = 0u;
-      if (base < S_scan) {
-#pragma unroll 1
-        for (int k = 0; k < 32 / G; ++k) {
-          const int j = base + k * G + sub;
-          const bool near = j < S_scan && slot_is_near(pool, batch, unit64, e, scn, j, px, py, n_upd, range, width);
-          word |= group_ballot<G>(gm, lane, near) << (k * G);
-        }
-      }
-      if (store && sub == 0) batch.nearby_mask[(long long)e * batch.mask_words + (base >> 5)] = word;
-    }
-#endif
     if (grid) {
       // uniform grid over the world's enclosing circles: only the polygons listed in the cells that the
       // detection disc's bounding box overlaps can be near; the exact test is the same
@@ -585,8 +566,9 @@ __device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned pari
       : "memory");
 }
 
-// BaseEnvironment._update (OBST) + Vessel.step (DYN) + Vessel.navigate + the culling stage, a
-// group of G lanes per env.  The scalar FP64 chains (RK step, PCHIP, navigation features) are
+// BaseEnvironment._update (OBST) + Vessel.step (DYN) + the path projection of Vessel.navigate, a
+// group of G lanes per env (k_nav_cull below, the same mapping, does the rest of Vessel.navigate and
+// the culling stage).  The scalar FP64 chains (RK step, PCHIP, navigation features) are
 // computed redundantly by the lanes of a group; the table searches (path projection, obstacle
 // slots) are split over them, which shortens the per-warp critical path ~G-fold and gives the
 // SM G times more warps to hide the remaining load latency with (thread-per-env had N/32 warps:
@@ -597,18 +579,9 @@ __device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned pari
 // the ~50 capsule tests per env then read shared memory instead of four dependent rounds of
 // global loads.  CTAs with mixed paths (or a path with more than AUV_PATH_STAGE_BLOCKS blocks)
 // search the global tables; the arithmetic is the same.
-#ifndef AUV_NAV_G
 #define AUV_NAV_G 4
-#endif
-#ifndef AUV_NAV_THREADS
 #define AUV_NAV_THREADS 128  // a multiple of 128: one 32-env sub-block (4 warps) per 128 threads
-#endif
-#ifndef AUV_NAV_MINB
 #define AUV_NAV_MINB (1024 / AUV_NAV_THREADS)  // 64 registers: 32 warps per SM (6 / 7 / 8 CTAs of 128: 0.106 / 0.101 / 0.096 ms)
-#endif
-#ifndef AUV_NAV_PHASE_SYNC
-#define AUV_NAV_PHASE_SYNC 0  // 1: __syncthreads between the phases, so that the warps of a CTA run the same code
-#endif
 constexpr int NAV_STAGE_SB = (AUV_PATH_STAGE_BLOCKS + AUV_PATH_SUPER - 1) / AUV_PATH_SUPER;
 constexpr int NAV_SUBBLOCKS = AUV_NAV_THREADS / 128;
 // shared memory of one sub-block: its path's capsule tables
@@ -618,11 +591,9 @@ struct __align__(16) NavStage {
   float4 sbc[NAV_STAGE_SB];
   float2 sba[NAV_STAGE_SB];
 };
-#ifndef AUV_NAV_SPLIT
-#define AUV_NAV_SPLIT 1  // two launches: k_vessel_nav stops after the projection, k_nav_cull does navigation + culling.
-                         // Same total kernel time as one launch (0.104 ms), but three kernels per env range
-                         // interleave better across the step's two streams: 0.180 -> 0.172 ms per step
-#endif
+// Two launches: k_vessel_nav stops after the projection, k_nav_cull does navigation + culling.  Same total
+// kernel time as one launch (0.104 ms), but three kernels per env range interleave better across the step's
+// two streams: 0.180 -> 0.172 ms per step
 template <bool DYN, bool OBST, int G>
 __global__ void __launch_bounds__(AUV_NAV_THREADS, AUV_NAV_MINB) k_vessel_nav(const __grid_constant__ AuvConfig cfg,
                                                                 const __grid_constant__ AuvPathBank paths,
@@ -691,7 +662,6 @@ __global__ void __launch_bounds__(AUV_NAV_THREADS, AUV_NAV_MINB) k_vessel_nav(co
       batch.step_counter[e] = step_counter;
     }
   }
-  if (AUV_NAV_PHASE_SYNC) __syncthreads();
   PathTabs T;
   if (staged) {
     mbar_wait(&s_bar[sbk], 0);
@@ -708,20 +678,13 @@ __global__ void __launch_bounds__(AUV_NAV_THREADS, AUV_NAV_MINB) k_vessel_nav(co
   int seg;
   const double s = project_group<G>(paths, h, T, y.x, y.y, prev_seg, lane, gm, seg, batch.status);
   AUV_CHECK(batch.status, seg >= 0 && seg < h.nseg && (!staged || (nblk <= AUV_PATH_STAGE_BLOCKS && nsb <= NAV_STAGE_SB)));
-  if (store && sub == 0) batch.prev_seg[e] = seg;
-  if (AUV_NAV_SPLIT) {  // hand the arclength to k_nav_cull
-    if (store && sub == 0) batch.nav[(long long)e * AUV_NAV_W + NAV_S] = s;
-    return;
+  if (store && sub == 0) {
+    batch.prev_seg[e] = seg;
+    batch.nav[(long long)e * AUV_NAV_W + NAV_S] = s;  // the arclength, handed to k_nav_cull
   }
-  if (AUV_NAV_PHASE_SYNC) __syncthreads();
-  navigate_env(cfg, paths, h, batch, pid, e, scn, s, y.x, y.y, y.psi, y.u, y.v, y.r,
-               obs_out ? obs_out + (long long)e * obs_dim : nullptr, store && sub == 0);
-  if (AUV_NAV_PHASE_SYNC) __syncthreads();
-  if (cfg.use_lidar)
-    cull_env_group<G>(cfg, pool, batch, unit64, windows_out, e, scn, y.x, y.y, y.psi, step_counter, n_upd, lane, gm, store);
 }
 
-// second half of the navigation kernel as its own launch (AUV_NAV_SPLIT builds): Vessel.navigate + the culling stage
+// second half of the navigation stage as its own launch: Vessel.navigate + the culling stage
 template <int G>
 __global__ void __launch_bounds__(128, 8) k_nav_cull(const __grid_constant__ AuvConfig cfg, const __grid_constant__ AuvPathBank paths,
                                                      const __grid_constant__ AuvScenarioPool pool,
@@ -763,15 +726,9 @@ __global__ void __launch_bounds__(128, 8) k_nav_cull(const __grid_constant__ Auv
 //      E envs at once, its outputs leave coalesced; finished envs are then auto-reset by a warp
 //      each (copy of the cached first observation)
 // ------------------------------------------------------------------------------------
-#ifndef AUV_LIDAR_THREADS
 #define AUV_LIDAR_THREADS 256
-#endif
-#ifndef AUV_LIDAR_RCAP
 #define AUV_LIDAR_RCAP 96  // records per shared-memory round
-#endif
-#ifndef AUV_LIDAR_MAX_ENVS
 #define AUV_LIDAR_MAX_ENVS 32  // envs per CTA (<= 32: one warp scans their record counts)
-#endif
 
 struct LidarArgs {
   AuvConfig cfg;
@@ -919,12 +876,7 @@ __device__ __forceinline__ void range_min(void* row, int i, float d, int slot) {
     atomicMin(reinterpret_cast<int*>(row) + i, __float_as_int(d));
 }
 
-#ifndef AUV_LIDAR_MINB
 #define AUV_LIDAR_MINB 5  // 48 registers (4 / 5 / 6 CTAs per SM: 0.0807 / 0.0767 / 0.101 ms)
-#endif
-#ifndef AUV_LIDAR_LONG_POLY
-#define AUV_LIDAR_LONG_POLY 1  // 0: tuning builds without the out-of-line long-polygon path (such polygons are flagged)
-#endif
 // A world polygon with more vertices than a warp's vertex stage holds, cast chain by chain
 // (consecutive chains share their end vertex).  Cold: land perimeters of thousands of vertices only.
 template <bool VEL>
@@ -1065,7 +1017,7 @@ __global__ void __launch_bounds__(AUV_LIDAR_THREADS, AUV_LIDAR_MINB) k_lidar(con
           if (nq > A.vmax) {
             // a world polygon with more vertices than the stage holds (land perimeters of any length): cast chain
             // by chain, out of line -- the hot loop below stays as small as it was without them
-            if (AUV_LIDAR_LONG_POLY && world)
+            if (world)
               cast_long_polygon<VEL>(reinterpret_cast<const double2*>(A.pool.world_verts) + q.vbase, nq, A.vmax, wverts,
                                      HAND(el, NAV_X), HAND(el, NAV_Y), HAND(el, NAV_COSPSI), HAND(el, NAV_SINPSI), cos_sin,
                                      q.ecx, q.ecy, q.rho, row, slot, lane, n1, n2, lo1, lo2, rangef);
@@ -1510,7 +1462,7 @@ __global__ void __launch_bounds__(AUV_SHIP_THREADS) k_obs_ship(const float* __re
 #define AUV_DELTA_THREADS 64
 #define AUV_DELTA_UNROLL 2
 // The kernel is bound by the host link, not by the SMs: it runs as a SMALL persistent grid (two
-// CTAs of 64 threads x 40 registers per SM by default: one fits into the registers five k_lidar
+// CTAs of 64 threads x 40 registers per SM: one fits into the registers five k_lidar
 // CTAs leave over) that strides over the range, so that its warps -- stalled on the link's write
 // queue most of the time -- leave the SMs to the step kernels of the next env range / env group
 // running beside it.  (One CTA per 256 quads, the first version, filled every
@@ -1788,10 +1740,7 @@ static int launch_vessel_nav(const AuvConfig* cfg, const AuvRayTable* rays, cons
   if (cnt < 0) cnt = batch->n_envs - e0;
   const int per_cta = AUV_NAV_THREADS / AUV_NAV_G;  // envs per CTA
   const int blocks = (cnt + per_cta - 1) / per_cta;
-#ifndef AUV_NAV_EXTRA_SMEM
-#define AUV_NAV_EXTRA_SMEM 0  // tuning: extra dynamic shared memory per CTA = a cap on resident CTAs per SM
-#endif
-  const size_t nsm = sizeof(auv::NavStage) * auv::NAV_SUBBLOCKS + AUV_NAV_EXTRA_SMEM;
+  const size_t nsm = sizeof(auv::NavStage) * auv::NAV_SUBBLOCKS;
   if (int rc = nav_configure(nsm)) return rc;
   const double2* unit = rays ? reinterpret_cast<const double2*>(rays->unit64) : nullptr;
   int* win = out ? out->windows : nullptr;
@@ -1804,13 +1753,10 @@ static int launch_vessel_nav(const AuvConfig* cfg, const AuvRayTable* rays, cons
     auv::k_vessel_nav<true, false, AUV_NAV_G><<<blocks, AUV_NAV_THREADS, nsm, s>>>(*cfg, *paths, *pool, *batch, unit, win, actions, obs, od, e0, e0 + cnt);
   else
     auv::k_vessel_nav<false, false, AUV_NAV_G><<<blocks, AUV_NAV_THREADS, nsm, s>>>(*cfg, *paths, *pool, *batch, unit, win, nullptr, obs, od, e0, e0 + cnt);
-  if (AUV_NAV_SPLIT) {
-    if (int rc = cuda_check(cudaGetLastError(), "k_vessel_nav")) return rc;
-    if (between != nullptr) cudaEventRecord(between, s);
-    auv::k_nav_cull<AUV_NAV_G><<<(cnt + 31) / 32, 128, 0, s>>>(*cfg, *paths, *pool, *batch, unit, win, obs, od, e0, e0 + cnt);
-    return cuda_check(cudaGetLastError(), "k_nav_cull");
-  }
-  return cuda_check(cudaGetLastError(), "k_vessel_nav");
+  if (int rc = cuda_check(cudaGetLastError(), "k_vessel_nav")) return rc;
+  if (between != nullptr) cudaEventRecord(between, s);
+  auv::k_nav_cull<AUV_NAV_G><<<(cnt + 31) / 32, 128, 0, s>>>(*cfg, *paths, *pool, *batch, unit, win, obs, od, e0, e0 + cnt);
+  return cuda_check(cudaGetLastError(), "k_nav_cull");
 }
 
 // the dynamic shared-memory opt-in of k_lidar is per device and per function; it is made once,
@@ -1957,7 +1903,7 @@ AuvPipeline* auv_pipeline_create(int n_streams) {
   p->n_streams = n_streams;
   p->gexec = nullptr;
   p->gkey = 0;
-  p->graph_state = getenv("AUV_B200_NO_GRAPH") ? -1 : 0;
+  p->graph_state = 0;
   bool ok = cudaEventCreateWithFlags(&p->fork, cudaEventDisableTiming) == cudaSuccess;
   int made = 0;
   for (; ok && made < n_streams; ++made) {
@@ -2060,7 +2006,7 @@ static int launch_obs_delta(const AuvConfig* cfg, const AuvStepOut* out, const A
     if (cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n_sm <= 0) n_sm = 148;
     sms[dev].store(n_sm);
   }
-  long long blocks = d->ctas > 0 ? d->ctas : 2 * n_sm;
+  long long blocks = 2 * n_sm;
   const long long need = (quads + AUV_DELTA_THREADS - 1) / AUV_DELTA_THREADS;
   if (blocks > need) blocks = need;
   if (blocks < 1) blocks = 1;
@@ -2148,7 +2094,7 @@ static int step_host_chunked(const AuvConfig* cfg, const AuvRayTable* rays, cons
       p->graph_state = 0;
       // one-time function attributes are set outside the capture
       if (int rc0 = lidar_configure(lidar_smem_bytes(cfg, pool))) return rc0;
-      if (int rc0 = nav_configure(sizeof(auv::NavStage) * auv::NAV_SUBBLOCKS + AUV_NAV_EXTRA_SMEM)) return rc0;
+      if (int rc0 = nav_configure(sizeof(auv::NavStage) * auv::NAV_SUBBLOCKS)) return rc0;
       cudaStream_t cs = p->st[1];
       cudaGraph_t graph = nullptr;
       int rc = 0;
@@ -2303,10 +2249,7 @@ int auv_step_timed(const AuvConfig* cfg, const AuvRayTable* rays, const AuvPathB
   cudaStream_t s = (cudaStream_t)stream;
   cudaEvent_t* e = t->ev + AUV_TIMER_EVENTS * slot;
   cudaEventRecord(e[0], s);
-  if (!AUV_NAV_SPLIT) cudaEventRecord(e[1], s);  // one navigation launch: interval 0 reads ~0, interval 1 is the kernel
-  if (int rc = launch_vessel_nav(cfg, rays, paths, pool, batch, out, actions, stream, 0, -1, true,
-                                 AUV_NAV_SPLIT ? e[1] : nullptr))
-    return rc;
+  if (int rc = launch_vessel_nav(cfg, rays, paths, pool, batch, out, actions, stream, 0, -1, true, e[1])) return rc;
   cudaEventRecord(e[2], s);
   if (int rc = launch_lidar(cfg, rays, paths, pool, batch, out, AUV_OBSERVE_STEP, stream)) return rc;
   return cuda_check(cudaEventRecord(e[3], s), "cudaEventRecord");

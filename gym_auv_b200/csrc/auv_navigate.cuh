@@ -167,16 +167,6 @@ constexpr int kSubPerBlk = AUV_PATH_BLOCK / AUV_PATH_SUB;  // sub-blocks of a bl
 // live node together instead of serialising over node indices.  The arg-min is lexicographic in
 // (distance, segment index), which is GEOS's "first minimum wins" independent of visiting order.
 // Every lane returns the same arclength; seg_out = the winning segment.
-#ifdef AUV_NOINLINE_PROJECT
-#define AUV_PROJECT_INLINE __noinline__
-#else
-#define AUV_PROJECT_INLINE __forceinline__
-#endif
-#ifdef AUV_NOINLINE_NAVIGATE
-#define AUV_NAVIGATE_INLINE __noinline__
-#else
-#define AUV_NAVIGATE_INLINE __forceinline__
-#endif
 // Upper bound of the distance without a previous segment (first step of an episode): pass A over
 // the superblock capsules, pass B over the block capsules of the superblocks that survive it.
 // Cold: kept out of line so that the hot path of the kernel stays small (the step kernel is
@@ -217,9 +207,9 @@ __device__ __noinline__ float project_cold_bound(const PathTabs& T, const int nb
 }
 
 template <int G>
-__device__ AUV_PROJECT_INLINE double project_group(const AuvPathBank& pb, const AuvPathHdr& h, const PathTabs& T,
-                                                   const double px, const double py, const int prev_seg,
-                                                   const int lane, const unsigned gm, int& seg_out, int* status = nullptr) {
+__device__ __forceinline__ double project_group(const AuvPathBank& pb, const AuvPathHdr& h, const PathTabs& T,
+                                                const double px, const double py, const int prev_seg,
+                                                const int lane, const unsigned gm, int& seg_out, int* status = nullptr) {
   constexpr int KB = AUV_PATH_SUPER / G;  // blocks of a superblock per lane
   constexpr int SPL = AUV_PATH_SUB > G ? AUV_PATH_SUB / G : 1;  // segments of a sub-block per lane
   static_assert(G >= kSubPerBlk, "one lane per sub-block of a block");
@@ -356,7 +346,7 @@ __device__ AUV_PROJECT_INLINE double project_group(const AuvPathBank& pb, const 
 // the LiDAR-independent part of the reward (rewarder.py:78-140,167-241).
 // `s` is the projected arclength (project_group); every lane of the env's group computes the
 // same scalars, `store` is true for the one lane that writes them.
-__device__ AUV_NAVIGATE_INLINE void navigate_env(const AuvConfig& cfg, const AuvPathBank& pb, const AuvPathHdr& h,
+__device__ __forceinline__ void navigate_env(const AuvConfig& cfg, const AuvPathBank& pb, const AuvPathHdr& h,
                                              const AuvBatch& batch, int pid, int e, int scn, const double s, double px,
                                              double py, double psi, double vu, double vv, double vr,
                                              float* __restrict__ obs_row, const bool store) {

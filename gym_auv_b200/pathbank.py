@@ -18,16 +18,15 @@ from __future__ import annotations
 from dataclasses import dataclass
 from typing import List, Sequence
 
-import os
-
 import numpy as np
 from scipy import interpolate
 
-PATH_BLOCK = int(os.environ.get("AUV_PATH_BLOCK", 32))  # must equal AUV_PATH_BLOCK in include/auv_b200.h (env override: tuning builds only)
-PATH_SUPER = int(os.environ.get("AUV_PATH_SUPER", 16))  # blocks per superblock, AUV_PATH_SUPER (env override: tuning builds only)
+from ._lib import PP_W
+
+PATH_BLOCK = 32  # segments per projection block, AUV_PATH_BLOCK in include/auv_b200.h
+PATH_SUPER = 16  # blocks per superblock, AUV_PATH_SUPER
 PATH_SUB = 8  # segments per sub-block, AUV_PATH_SUB
 N_KNOTS = 1000
-PP_W = 12  # AUV_PP_W
 HDR_DTYPE = np.dtype([("v0", "<i4"), ("nseg", "<i4"), ("b0", "<i4"), ("s0", "<i4"), ("ox", "<f8"), ("oy", "<f8"),
                       ("length", "<f8"), ("end_x", "<f8"), ("end_y", "<f8"), ("extent", "<f8")])  # AuvPathHdr
 

@@ -13,7 +13,6 @@ PyTorch is used for device memory and streams only; all arithmetic is in
 from __future__ import annotations
 
 import ctypes as C
-import os
 import time
 from typing import Dict, Optional
 
@@ -940,7 +939,7 @@ class AUVVecEnv:
                     p["shadow"] = torch.zeros((N, self.obs_dim), dtype=torch.float32, device=self.device)
                     p["shipped"] = torch.zeros(1, dtype=torch.int64, device=self.device)
                     p["delta"] = _lib.AuvDelta(p["obs"].data_ptr(), p["shadow"].data_ptr(), p["shipped"].data_ptr(),
-                                               self.delta_gran, int(os.environ.get("AUV_B200_DELTA_CTAS", "0")))
+                                               self.delta_gran)
         return self._pinned
 
     @property

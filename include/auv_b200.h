@@ -61,12 +61,8 @@ extern "C" {
 
 #define AUV_MAX_RAYS 1024
 #define AUV_MAX_OBSTACLES 1024 /* moving + static slots per env */
-#ifndef AUV_PATH_BLOCK
 #define AUV_PATH_BLOCK 32     /* polyline segments per projection block */
-#endif
-#ifndef AUV_PATH_SUPER
 #define AUV_PATH_SUPER 16     /* blocks per projection superblock (8 / 16 / 32 swept: profiles/r1j_variants.txt) */
-#endif
 #define AUV_PATH_SUB 8        /* polyline segments per sub-block (a block holds AUV_PATH_BLOCK / AUV_PATH_SUB of them) */
 #define AUV_NAV_W 24          /* doubles per env in AuvBatch.nav */
 #define AUV_REC_BYTES 80      /* bytes per obstacle record in AuvBatch.rec */
@@ -77,10 +73,8 @@ extern "C" {
 #define AUV_STATUS_BOUNDS 16 /* -DAUV_DEBUG_BOUNDS builds only: an index check of a step kernel failed */
 #define AUV_STATUS_POLY_TOO_LARGE 4 /* a world polygon has more than AUV_MAX_POLY_VERTS vertices: it was skipped */
 #define AUV_STATUS_GEN_LAND_BLOCKED 32 /* scenario generator: no vessel start clear of land in 4096 draws (last one kept) */
-#ifndef AUV_PATH_STAGE_BLOCKS
-#define AUV_PATH_STAGE_BLOCKS 512
-#endif                            /* paths with at most this many projection blocks (~1.6 km) are searched from a
-                                     shared-memory copy of their capsule tables (one bulk async copy per CTA) */
+#define AUV_PATH_STAGE_BLOCKS 512 /* paths with at most this many projection blocks (~1.6 km) are searched from a
+                                    shared-memory copy of their capsule tables (one bulk async copy per CTA) */
 #define AUV_PP_W 12           /* doubles per PCHIP piece record in AuvPathBank.pp */
 
 /* gym_auv/config.py field names (EpisodeConfig/SimulationConfig/VesselConfig).  POD. */
@@ -388,7 +382,7 @@ AuvPipeline* auv_pipeline_create(int n_streams);
 void auv_pipeline_destroy(AuvPipeline* p);
 /* 1: auv_step_host_chunked replays an instantiated CUDA graph (one launch per step; re-captured
  * when an argument changes), 0: nothing captured yet, -1: direct submission (capture was not
- * possible, or AUV_B200_NO_GRAPH is set in the environment). */
+ * possible). */
 int auv_pipeline_graph_state(const AuvPipeline* p);
 int auv_step_chunked(const AuvConfig* cfg, const AuvRayTable* rays, const AuvPathBank* paths,
                      const AuvScenarioPool* pool, AuvBatch* batch, const float* actions,
@@ -444,7 +438,7 @@ typedef struct AuvDelta {
   float* shadow;                /* [N][obs_dim] device, 16 B aligned                       */
   unsigned long long* shipped;  /* [1] device, cumulative chunks stored (NULL: not counted) */
   int32_t gran;                 /* floats per chunk: 8, 16 or 32                           */
-  int32_t ctas;                 /* CTAs of the (link-bound, persistent) kernel; 0 = two per SM */
+  int32_t reserved0;            /* ignored (set to 0)                                      */
 } AuvDelta;
 int auv_step_host_delta_submit(const AuvConfig* cfg, const AuvRayTable* rays, const AuvPathBank* paths,
                                const AuvScenarioPool* pool, AuvBatch* batch, const float* actions_host,

@@ -174,6 +174,22 @@ def test_binding_layout_and_version(built_lib):
     assert lib.auv_obs_dim(ctypes.byref(cfg)) == 6
 
 
+def test_python_constants_equal_the_header_defines():
+    """The host code sizes and indexes device tables with Python copies of the header's constants (pathbank
+    builds the capsule tables the kernels search by AUV_PATH_BLOCK / SUPER / SUB): each copy must equal its
+    #define, and every status bit must have one."""
+    from gym_auv_b200 import _lib, pathbank
+
+    hdr = open(os.path.join(ROOT, "include", "auv_b200.h")).read()
+    defines = {k: int(v) for k, v in re.findall(r"^#define (AUV_\w+) +\(?(-?\d+)\)?", hdr, flags=re.M)}
+    status = sorted(k[len("AUV_"):] for k in defines if k.startswith("AUV_STATUS_"))
+    assert status and status == sorted(k for k in vars(_lib) if k.startswith("STATUS_"))
+    mirrors = {f"AUV_{k}": getattr(_lib, k) for k in status + ["ABI_VERSION", "REC_BYTES", "MAX_POLY_VERTS", "NAV_W", "PP_W",
+                                                             "PATH_STAGE_BLOCKS"]}
+    mirrors.update(AUV_PATH_BLOCK=pathbank.PATH_BLOCK, AUV_PATH_SUPER=pathbank.PATH_SUPER, AUV_PATH_SUB=pathbank.PATH_SUB)
+    assert mirrors == {k: defines.get(k) for k in mirrors}
+
+
 def test_scenario_template_is_the_input_of_gpu_generation():
     scn = S.moving_obstacles_template(64, 5, 3, seed=1, n_paths=4)
     assert scn.n_scenarios == 64 and scn.k_moving == 5 and scn.k_static == 3 and len(scn.waypoints) == 4
