@@ -35,6 +35,22 @@ STAT_NAMES = [
     "steps",
 ]
 
+# render palette (0xRRGGBB) and frame constants, AUV_RGB_* / AUV_RENDER_* in include/auv_b200.h (rule at AuvRender)
+RGB_OWNSHIP = 0xF2C12E
+RGB_RAY_HIT = 0xE4572E
+RGB_RAY_CLEAR = 0x4F7CAC
+RGB_MOVING = 0xD7263D
+RGB_STATIC = 0x8E5572
+RGB_GOAL = 0x3BB273
+RGB_PATH = 0xF4F4F4
+RGB_LAND = 0x6B8F3E
+RGB_SEA = 0x0B2545
+RENDER_SHIP_MIN_PX = 8
+RENDER_GOAL_PX = 4
+RENDER_PATH_HALF_PX = 1.0
+RENDER_RAY_HALF_PX = 0.5
+RENDER_MAX_DIM = 4096
+
 OBSERVE_STEP = 0
 OBSERVE_RESET = 1
 REWARDER_IDS = {"colav": 0, "pathfollow": 1}
@@ -249,6 +265,11 @@ class AuvDelta(C.Structure):
     _fields_ = [("obs_host", _vp), ("shadow", _vp), ("shipped", _vp), ("gran", C.c_int32), ("reserved0", C.c_int32)]
 
 
+class AuvRender(C.Structure):
+    _fields_ = [("count", C.c_int32), ("width", C.c_int32), ("height", C.c_int32), ("reserved0", C.c_int32),
+                ("env_ids", _vp), ("half_width", C.c_double)]
+
+
 EXPORTS = [
     "auv_abi_version",
     "auv_sizeof",
@@ -283,6 +304,7 @@ EXPORTS = [
     "auv_compact_expand",
     "auv_pathbank_build",
     "auv_random_curve_waypoints",
+    "auv_render",
 ]
 
 _lib = None
@@ -357,6 +379,8 @@ def load():
     lib.auv_compact_expand.argtypes = [P(AuvConfig), C.c_int, P(AuvCompact), _vp, _vp, C.c_int]
     lib.auv_pathbank_build.argtypes = [_vp, _vp, _vp, C.c_int, P(AuvPathBuild), _vp, _vp]
     lib.auv_random_curve_waypoints.argtypes = [C.c_uint64, C.c_uint32, C.c_double, _vp, C.c_int, _vp, _vp, _vp]
+    lib.auv_render.argtypes = [P(AuvConfig), P(AuvRayTable), P(AuvPathBank), P(AuvScenarioPool), P(AuvBatch), _vp,
+                               P(AuvRender), _vp, _vp]
     lib.auv_timer_create.argtypes = [C.c_int]
     lib.auv_timer_create.restype = _vp
     lib.auv_timer_destroy.argtypes = [_vp]
@@ -372,7 +396,7 @@ def load():
         raise AuvLibraryError(f"ABI mismatch: library {ver}, binding {ABI_VERSION}; rebuild")
     lib.auv_sizeof.argtypes = [C.c_int]
     for i, st in enumerate([AuvConfig, AuvRayTable, AuvPathBank, AuvScenarioPool, AuvBatch, AuvStepOut, AuvGenParams,
-                            AuvPathHdr, AuvRefreshScratch, AuvCompact, AuvPathBuild, AuvDelta, AuvTracks]):
+                            AuvPathHdr, AuvRefreshScratch, AuvCompact, AuvPathBuild, AuvDelta, AuvTracks, AuvRender]):
         if lib.auv_sizeof(i) != C.sizeof(st):
             raise AuvLibraryError(f"struct layout mismatch for {st.__name__}: C {lib.auv_sizeof(i)} vs ctypes {C.sizeof(st)}")
     _lib = lib

@@ -140,6 +140,32 @@ class B200VecEnv:
             return self.seed(*args, **kwargs)
         raise AttributeError(f"B200VecEnv has no per-env method {method_name!r}")
 
+    def get_images(self, indices: Optional[Sequence[int]] = None, half_width: Optional[float] = None) -> List[np.ndarray]:
+        """``VecEnv.get_images``: one ``np.uint8`` (400, 400, 3) top-down frame per env (``AUVVecEnv.render``;
+        ``half_width`` defaults to ``config.vessel.render_distance`` and must be given when that is not a number).
+        The default is the first ``min(num_envs, 16)`` envs, not all of them: video recorders call this every
+        step, and frames of 65536 envs would be 31 GB; a 4 x 4 grid is what a person can look at."""
+        idx = list(range(min(self.num_envs, 16))) if indices is None else ([indices] if isinstance(indices, int) else list(indices))
+        frames = self.impl.render(idx, half_width=half_width).cpu().numpy()
+        return [f for f in frames]
+
+    def render(self, mode: str = "rgb_array", indices: Optional[Sequence[int]] = None,
+               half_width: Optional[float] = None) -> np.ndarray:
+        """``VecEnv.render``: the ``get_images`` frames tiled into one image, ``ceil(sqrt(n))`` columns, row by
+        row, black where the grid has no frame.  Only ``"rgb_array"``: there is no window."""
+        if mode != "rgb_array":
+            raise NotImplementedError(f"render mode {mode!r}: only 'rgb_array' is supported (there is no window)")
+        imgs = self.get_images(indices, half_width=half_width)
+        n = len(imgs)
+        cols = int(np.ceil(np.sqrt(n)))
+        rows = (n + cols - 1) // cols
+        h, w, _ = imgs[0].shape
+        out = np.zeros((rows * h, cols * w, 3), dtype=np.uint8)
+        for k, img in enumerate(imgs):
+            r, c = divmod(k, cols)
+            out[r * h:(r + 1) * h, c * w:(c + 1) * w] = img
+        return out
+
     def episode_stats(self, reduce: bool = True):
         return self.impl.episode_stats(reduce=reduce)
 

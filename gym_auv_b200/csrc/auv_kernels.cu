@@ -22,6 +22,7 @@
 //                      twins also record the episode tracks of AuvStepOut.tracks    FP32 issue
 //   k_obstacle_update / k_vessel_step / k_reset   staged entry points
 //   k_pool_pack, k_obstacle_state                  pool packing / obstacle state read-back
+//   k_render           top-down RGB frames of a sample of the batch (auv_render.cuh)
 //   k_fma_probe        FP32 FMA peak micro-benchmark (roofline denominator)
 //
 // Precision plan: everything cheap and threshold-sensitive is FP64 (vessel state, RK step,
@@ -1541,6 +1542,8 @@ __global__ void __launch_bounds__(256) k_fma_probe(float* sink, int iters) {
 
 }  // namespace auv
 
+#include "auv_render.cuh"
+
 // ======================================================================================
 // C ABI
 // ======================================================================================
@@ -1581,6 +1584,7 @@ int auv_sizeof(int which) {
     case 10: return (int)sizeof(AuvPathBuild);
     case 11: return (int)sizeof(AuvDelta);
     case 12: return (int)sizeof(AuvTracks);
+    case 13: return (int)sizeof(AuvRender);
     default: return AUV_EINVAL;
   }
 }
@@ -2490,6 +2494,51 @@ int auv_fma_probe(float* sink, int blocks, int threads, int iters, void* stream,
   auv::k_fma_probe<<<blocks, threads, 0, (cudaStream_t)stream>>>(sink, iters);
   if (flops_out) *flops_out = 2.0 * 8.0 * (double)iters * (double)blocks * (double)threads;
   return cuda_check(cudaGetLastError(), "k_fma_probe");
+}
+
+int auv_render(const AuvConfig* cfg, const AuvRayTable* rays, const AuvPathBank* paths, const AuvScenarioPool* pool,
+               const AuvBatch* batch, const float* obs, const AuvRender* r, uint8_t* frames, void* stream) {
+  if (!cfg || !rays || !paths || !pool || !batch || !r || !frames || !r->env_ids)
+    return set_err(AUV_EINVAL, "auv_render: NULL argument");
+  if (int rc = check_cfg(cfg)) return rc;
+  if (cfg->use_lidar && (!obs || !rays->cos_sin)) return set_err(AUV_EINVAL, "auv_render: obs / rays.cos_sin is NULL with use_lidar");
+  if (r->count < 1) return set_err(AUV_EINVAL, "auv_render: count must be >= 1");
+  if (r->width < 1 || r->width > AUV_RENDER_MAX_DIM || r->height < 1 || r->height > AUV_RENDER_MAX_DIM)
+    return set_err(AUV_EINVAL, "auv_render: width and height must be in 1..4096");
+  if (!(isfinite(r->half_width) && r->half_width > 0.0)) return set_err(AUV_EINVAL, "auv_render: half_width must be finite and > 0");
+  if (batch->n_envs <= 0) return set_err(AUV_EINVAL, "n_envs must be > 0");
+  if (!batch->state || !batch->scn_id || !batch->obst_steps || !batch->env_pid)
+    return set_err(AUV_EINVAL, "auv_render: batch.state / scn_id / obst_steps / env_pid is NULL");
+  if (!paths->hdr || !paths->poly_xy || !paths->blk_chord || !paths->blk_dev)
+    return set_err(AUV_EINVAL, "auv_render: path bank arrays are NULL");
+  if (pool->k_moving < 0 || pool->k_static < 0 || pool->n_world < 0) return set_err(AUV_EINVAL, "negative slot count");
+  if (pool->k_static > 0 && (!pool->st_rec || !rays->unit64)) return set_err(AUV_EINVAL, "auv_render: pool.st_rec / rays.unit64 is NULL");
+  if (int rc = check_pool_tracks(pool, batch)) return rc;
+  if (pool->k_moving > 0 && (pool->linear_tracks ? !pool->mov_disp0 : !pool->mov_width))
+    return set_err(AUV_EINVAL, "auv_render: pool.mov_disp0 / mov_width is NULL");
+  if (pool->n_world > 0) {
+    if (!pool->world_circle || !pool->world_voff || !pool->world_verts) return set_err(AUV_EINVAL, "world arrays are NULL");
+    if (pool->world_cell_off &&
+        (!pool->world_cell_items || pool->world_grid_nx <= 0 || pool->world_grid_ny <= 0 || !(pool->world_grid_cell > 0.0)))
+      return set_err(AUV_EINVAL, "world grid: NULL items or empty grid");
+  }
+  auv::RenderArgs a;
+  a.cfg = *cfg;
+  a.rays = *rays;
+  a.paths = *paths;
+  a.pool = *pool;
+  a.batch = *batch;
+  a.obs = obs;
+  a.env_ids = r->env_ids;
+  a.frames = frames;
+  a.half_width = r->half_width;
+  a.obs_dim = auv_obs_dim(cfg);
+  a.width = r->width;
+  a.height = r->height;
+  a.tiles_x = (r->width + AUV_RENDER_TILE - 1) / AUV_RENDER_TILE;
+  const int tiles_y = (r->height + AUV_RENDER_TILE - 1) / AUV_RENDER_TILE;
+  auv::k_render<<<dim3((unsigned)r->count, (unsigned)(a.tiles_x * tiles_y)), AUV_RENDER_THREADS, 0, (cudaStream_t)stream>>>(a);
+  return cuda_check(cudaGetLastError(), "k_render");
 }
 
 }  // extern "C"

@@ -14,8 +14,10 @@ counterpart of setting ``self.vessel/self.path/self.obstacles``, environment.py:
 holding one scenario -- or, via ``_generate_block(n)``, the scenarios of the next n episodes:
 the facade keeps ONE AUVVecEnv (device tables, path bank, reset cache) alive for the whole
 block and moves from scenario to scenario with ``reset_envs``; it is rebuilt only when the
-block is used up.  Rendering is out of scope (SURVEY.md section 2 #14-15):
-``renderer`` must be None.
+block is used up.  ``render(mode="rgb_array")`` returns a top-down RGB frame of the env drawn on the GPU
+(``AUVVecEnv.render``; a visual tap, no parity with the reference's pygame renderer is claimed).  There is
+no window: "human" mode and the 2-D / 3-D viewers stay out of scope (SURVEY.md section 2 #14-15), so the
+``renderer`` constructor argument must be None.
 """
 from __future__ import annotations
 
@@ -41,7 +43,7 @@ REWARDER_PARAMS = {  # rewarder.py:56-70, 143-159
 class AUVEnv:
     """Base class; subclasses provide ``_generate()`` (see ``scenario_env``)."""
 
-    metadata = {"render.modes": []}
+    metadata = {"render.modes": ["rgb_array"]}
     scenario_name = ""
     block_size = 64  # episodes generated (and uploaded) at a time by families that implement _generate_block
 
@@ -168,8 +170,12 @@ class AUVEnv:
     def close(self):
         self._vec = None
 
-    def render(self, mode="rgb_array", **kwargs):
-        raise NotImplementedError("rendering is outside the B200 step path (SURVEY.md section 2 #14)")
+    def render(self, mode="rgb_array", width: int = 400, height: int = 400, half_width=None):
+        """``np.uint8`` (height, width, 3): the env as its last step or reset left it, north up, centred on the
+        vessel (``AUVVecEnv.render``; ``half_width`` defaults to ``config.vessel.render_distance``)."""
+        if mode != "rgb_array":
+            raise NotImplementedError(f"render mode {mode!r}: only 'rgb_array' is supported (there is no window)")
+        return self._vec.render([0], width=width, height=height, half_width=half_width)[0].cpu().numpy()
 
     def _format_obs(self, obs):
         if isinstance(obs, dict):  # the batched env already split it (AUVVecEnv.observation_dict)

@@ -1000,6 +1000,48 @@ class AUVVecEnv:
             )
         return self._out["obs"]
 
+    # ------------------------------------------------------------------ rendering
+    def render(self, env_ids, width: int = 400, height: int = 400, half_width: Optional[float] = None) -> torch.Tensor:
+        """Top-down RGB frames of envs ``env_ids`` as their last step or reset left them: a CUDA ``uint8`` tensor
+        [K, height, width, 3], north up, centred on each vessel, ``2 half_width / width`` metres per pixel (the
+        frame rule is stated at ``AuvRender`` in include/auv_b200.h).  A visual tap: no parity with the
+        reference's pygame renderer is claimed.  Enqueued on the current stream (auv_render, kernel k_render)
+        with no host synchronisation; it reads env state and the device observation rows only -- every step
+        path (``step``, ``step_host``, ``step_async`` / ``step_wait`` with each host transfer) computes those
+        rows on the device before any copy, so the rays are the last step's.
+
+        ``env_ids``: at least one id; ints on the host (checked: ValueError when out of range) or an int CUDA
+        tensor (not read back; a frame whose id is out of range comes out all zeros).  ``half_width`` defaults to
+        ``config.vessel.render_distance`` when that is a number.  RuntimeError between ``step_async()`` and
+        ``step_wait()``: the step in flight is writing what a frame would show."""
+        if getattr(self, "_async_pending", False):
+            raise RuntimeError("render() between step_async() and step_wait(): call step_wait() first")
+        if half_width is None:
+            rd = self.config.vessel.render_distance
+            if isinstance(rd, bool) or not isinstance(rd, (int, float)):
+                raise ValueError(f"config.vessel.render_distance is {rd!r}, not a number: pass half_width")
+            half_width = float(rd)
+        if isinstance(env_ids, torch.Tensor) and env_ids.is_cuda:
+            # ids outside [0, N) become -1 before the narrowing to int32, so that none can wrap into the batch
+            t = env_ids.to(device=self.device).reshape(-1)
+            ids = torch.where((t >= 0) & (t < self.num_envs), t, torch.full_like(t, -1)).to(torch.int32).contiguous()
+        else:
+            host = np.asarray(env_ids.cpu() if isinstance(env_ids, torch.Tensor) else env_ids, dtype=np.int64).reshape(-1)
+            if host.size and (host.min() < 0 or host.max() >= self.num_envs):
+                raise ValueError(f"env ids must be in [0, {self.num_envs}), got {host.tolist()}")
+            # pinned + non_blocking: the copy is ordered on the stream without waiting for it
+            ids = torch.from_numpy(host.astype(np.int32)).pin_memory().to(self.device, non_blocking=True)
+        K = int(ids.numel())
+        if K == 0:
+            raise ValueError("render() needs at least one env id")
+        frames = torch.empty((K, int(height), int(width), 3), dtype=torch.uint8, device=self.device)
+        desc = _lib.AuvRender(K, int(width), int(height), 0, ids.data_ptr(), float(half_width))
+        cfg, rays, paths, pool, batch = self._refs()
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.auv_render(cfg, rays, paths, pool, batch, C.c_void_p(self._out["obs"].data_ptr()),
+                                           C.byref(desc), C.c_void_p(frames.data_ptr()), self._stream()), "auv_render")
+        return frames
+
     # ------------------------------------------------------------------ episode tracks (record_tracks)
     def _track_slot(self, i: int) -> Optional[int]:
         if self._tracks is None:

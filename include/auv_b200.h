@@ -336,7 +336,7 @@ typedef struct AuvStepOut {
 int auv_abi_version(void);
 /* sizeof of the ABI structs, in declaration order (0 AuvConfig, 1 AuvRayTable, 2 AuvPathBank,
  * 3 AuvScenarioPool, 4 AuvBatch, 5 AuvStepOut, 6 AuvGenParams, 7 AuvPathHdr, 8 AuvRefreshScratch, 9 AuvCompact,
- * 10 AuvPathBuild, 11 AuvDelta, 12 AuvTracks) so a binding
+ * 10 AuvPathBuild, 11 AuvDelta, 12 AuvTracks, 13 AuvRender) so a binding
  * can verify its layout. */
 int auv_sizeof(int which);
 const char* auv_last_error(void);
@@ -576,6 +576,57 @@ int auv_pool_pack(const AuvConfig* cfg, const AuvScenarioPool* pool, const int32
  * pool.linear_tracks they are evaluated from the closed form, otherwise copied from AuvBatch. */
 int auv_obstacle_state(const AuvConfig* cfg, const AuvScenarioPool* pool, const AuvBatch* batch, double* pos,
                        double* disp, double* counter, void* stream);
+/* Top-down RGB frames of live envs (a visual tap for trainers and video recorders; no parity with the
+ * reference's pygame renderer is claimed).  A frame is uint8 [height][width][3] RGB, contiguous; the
+ * count frames are [count][height][width][3].  Frame f shows env env_ids[f] as its last step or reset left
+ * it; rendering reads env state only.
+ *   Camera: north-up, centred on the vessel (state x = north, y = east), square pixels of
+ *   s = 2 half_width / width metres.  The centre of pixel (row r, column c), 0-based, row 0 at the top, lies
+ *   dx = (height/2 - r - 0.5) s north and dy = (c + 0.5 - width/2) s east of the vessel.
+ *   Coverage: a pixel takes the colour of the FIRST layer below whose shape contains its centre (no
+ *   anti-aliasing, no blending):
+ *     1 own-ship   filled c_pent pentagon (the VesselObstacle body), area centroid at (x, y), rotated by psi,
+ *                  width max(vessel_width, AUV_RENDER_SHIP_MIN_PX s)                        AUV_RGB_OWNSHIP
+ *     2 LiDAR rays (use_lidar only) capsule of half-width AUV_RENDER_RAY_HALF_PX s around the segment from
+ *                  (x, y) to (x, y) + d_i (cos(psi + a_i), sin(psi + a_i)), a_i the ray table's body angle,
+ *                  d_i from the closeness c_i = obs[e][6 + i] (channel 0): (1 + range)^(1 - c_i) - 1 with
+ *                  sensor_log_transform, (1 - c_i) range without, range when c_i = 0.  AUV_RGB_RAY_HIT
+ *                  where a ray with c_i > 0 covers the pixel, else AUV_RGB_RAY_CLEAR
+ *     3 moving obstacles  filled VesselObstacle pentagon at the env's current obstacle state  AUV_RGB_MOVING
+ *     4 static circles    filled n-gon buffer(r).boundary.simplify(0.3), ngon_sides(r) vertices  AUV_RGB_STATIC
+ *     5 goal       disc of radius AUV_RENDER_GOAL_PX s around Path.end (AuvPathHdr.end_x / end_y)  AUV_RGB_GOAL
+ *     6 path       capsule of half-width AUV_RENDER_PATH_HALF_PX s around the env's 0.1 m polyline  AUV_RGB_PATH
+ *     7 land       world polygons, even-odd rule on the closed ring (a polygon of more than
+ *                  AUV_MAX_POLY_VERTS vertices is not drawn: the step skips it too)           AUV_RGB_LAND
+ *     8 sea        everything else                                                              AUV_RGB_SEA
+ *   Empty slots (width / radius <= 0) draw nothing.  A frame whose env id is outside [0, n_envs) is all
+ *   zeros (nothing of the batch is read for it). */
+#define AUV_RGB_OWNSHIP 0xF2C12Eu
+#define AUV_RGB_RAY_HIT 0xE4572Eu
+#define AUV_RGB_RAY_CLEAR 0x4F7CACu
+#define AUV_RGB_MOVING 0xD7263Du
+#define AUV_RGB_STATIC 0x8E5572u
+#define AUV_RGB_GOAL 0x3BB273u
+#define AUV_RGB_PATH 0xF4F4F4u
+#define AUV_RGB_LAND 0x6B8F3Eu
+#define AUV_RGB_SEA 0x0B2545u
+#define AUV_RENDER_SHIP_MIN_PX 8   /* own-ship width at least this many pixels                  */
+#define AUV_RENDER_GOAL_PX 4       /* goal disc radius, pixels                                  */
+#define AUV_RENDER_PATH_HALF_PX 1.0 /* path stroke half-width, pixels                            */
+#define AUV_RENDER_RAY_HALF_PX 0.5 /* ray stroke half-width, pixels                             */
+#define AUV_RENDER_MAX_DIM 4096    /* width and height are 1 .. AUV_RENDER_MAX_DIM              */
+typedef struct AuvRender {
+  int32_t count;           /* K >= 1 frames                                                   */
+  int32_t width, height;   /* pixels, 1 .. AUV_RENDER_MAX_DIM                                 */
+  int32_t reserved0;       /* ignored (set to 0)                                              */
+  const int32_t* env_ids;  /* device [count] env of each frame                                */
+  double half_width;       /* metres from the vessel to the left / right frame edge, finite > 0 */
+} AuvRender;
+/* Renders the frames into `frames` (device, count * height * width * 3 bytes) on `stream`, without
+ * synchronising.  obs is the device [N][obs_dim] observation buffer the last step or reset wrote (AuvStepOut.obs;
+ * may be NULL without use_lidar).  Bad arguments return AUV_EINVAL before any device work. */
+int auv_render(const AuvConfig* cfg, const AuvRayTable* rays, const AuvPathBank* paths, const AuvScenarioPool* pool,
+               const AuvBatch* batch, const float* obs, const AuvRender* r, uint8_t* frames, void* stream);
 /* Measured FP32 FMA peak helper (roofline denominator): runs `iters` dependent FMAs per
  * thread on a full grid; the caller times it with CUDA events. Returns flop count. */
 int auv_fma_probe(float* sink, int blocks, int threads, int iters, void* stream,
